@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            (N > 1: launched by torchrun, one rank per GPU)
     python bench.py --impl reference ...                       (the reference CPU path on the host cores)
+    python bench.py ... --dump-outputs DIR                     (also write a fixed sample of the last timed step's outputs as DIR/*.npy)
 
 A "step" is one pass of the fused observation chain (brightness/contrast -> HSV colour masks || 3-channel Canny ->
 merge -> /255 float tensor) over one batch of synthetic 120x160 frames, sharded by env index with no data-path
@@ -57,6 +58,8 @@ NOTES = {
 
 
 _REAL_STDOUT = None
+# --dump-outputs sample sizes: 32 frames of 240x320 with u8 and f32 outputs, both written as float32, are 59 MB (under 64 MB)
+DUMP_FRAMES, DUMP_CARS = 32, 65536
 
 
 def load_track(name: str):
@@ -73,6 +76,29 @@ def emit(line: dict):
     if _REAL_STDOUT is not None:
         os.dup2(_REAL_STDOUT, 1)
     print(json.dumps(line), flush=True)
+
+
+def dump_outputs(out_dir, start, groups):
+    """Writes a fixed, seeded sample of rows of each output as out_dir/<name>.npy: int32 and float64 outputs as float64, the others as
+    float32 (exact for u8 and f32).  groups: (index name, sample size, {name: device tensor with one row per frame or car}); the global
+    index of each sampled row goes to out_dir/<index name>.npy, so that two builds can be compared output for output."""
+    import numpy as np
+    import torch
+    arrays = {}
+    for seed, (index_name, k, outputs) in enumerate(groups):
+        outputs = {name: t for name, t in outputs.items() if t is not None}
+        if not outputs:
+            continue
+        n = next(iter(outputs.values())).shape[0]
+        rows = np.arange(n) if n <= k else np.sort(np.random.default_rng(seed).choice(n, k, replace=False))
+        arrays[index_name] = (rows + start).astype(np.float64)
+        for name, t in outputs.items():
+            a = t.index_select(0, torch.from_numpy(rows).to(t.device)).cpu().numpy()
+            arrays[name] = a.astype(np.float64 if a.dtype in (np.float64, np.int32) else np.float32)
+    assert sum(a.nbytes for a in arrays.values()) <= 64 * 10**6
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def read_tensor_peak():
@@ -586,7 +612,11 @@ def main():
     ap.add_argument("--no-others", action="store_true")
     ap.add_argument("--no-blocks", action="store_true", help="skip the 240x320 / 1M-frame pipeline / statistics blocks")
     ap.add_argument("--quick", action="store_true", help="the headline step only (kernel iteration, ncu)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write a fixed sample of what the last step computed "
+                                                          "(rank 0's shard) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the CUDA path (--impl b200)")
     if args.quick:
         args.no_cpu_baseline = args.no_e2e = args.no_others = args.no_blocks = True
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
@@ -648,21 +678,24 @@ def main():
         return c
 
     def cars_step(c):
-        c["trk"].locate_device(c["xyz"])
+        idx, seg = c["trk"].locate_device(c["xyz"])
         s_, t_, b_, _ = c["spd"].control_device(c["cur"], c["st"], c["ms"])
         c["clock"] += 0.05
-        c["mux"].mux_device(c["mode"], c["usr"], torch.stack([s_, t_, b_]), c["clock"], speed=c["cur"], params=c["prm"])
+        mux = c["mux"].mux_device(c["mode"], c["usr"], torch.stack([s_, t_, b_]), c["clock"], speed=c["cur"], params=c["prm"])
+        return {"loc_index": idx, "loc_segment": seg, "ai_steering": s_, "ai_throttle": t_, "ai_breaking": b_,
+                "mux_steering": mux[0], "mux_throttle": mux[1], "mux_breaking": mux[2]}
 
     def close_cars(c):
         for k in ("trk", "spd", "mux"):
             c[k].onShutdown()
 
     cars = make_cars(end - start, 4 + rank) if args.workload == "full_pipeline_1M_over_8" else None
+    last_cars = {}
 
     def step():
         comp.process_device(batch, out_u8=out_u8, out_f32=out_f32, want_u8=want_u8, want_f32=want_f32)
         if cars is not None:
-            cars_step(cars)
+            last_cars.update(cars_step(cars))
 
     # ---- headline: K steps of the workload ------------------------------------------------------------------------------------
     for _ in range(args.warmup):
@@ -685,6 +718,9 @@ def main():
     ms_per_step = elapsed_ms / args.steps
     total_frames = frames * world
     value = total_frames / (ms_per_step * 1e-3)
+    if args.dump_outputs and rank == 0:              # before the blocks below write into out_u8 / out_f32 again (tub mode: JPEG-decoded frames)
+        dump_outputs(args.dump_outputs, start, [("frame_index", DUMP_FRAMES, {"cam_processed_img": out_u8, "cam_normalised_img": out_f32}),
+                                                ("car_index", DUMP_CARS, last_cars)])
 
     # ---- the same step with the per-step statistics ON: counters in the kernel + the system's only collective (a 192-byte all-reduce over
     # NCCL) every step, inside the timed region (north_star: "NCCL used only to gather per-step statistics") ------------------------------

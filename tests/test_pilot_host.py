@@ -113,12 +113,18 @@ def test_weight_file_round_trip(tmp_path):
 
 
 def test_pilot_without_a_gpu_fails_loudly():
-    if torch.cuda.is_available():
-        pytest.skip("needs a box without a GPU")
-    from triton_racer_sim_b200 import _native as nat
-    from triton_racer_sim_b200.pilot import ModelType, PilotNet
-    with pytest.raises((nat.NativeError, RuntimeError)):
-        PilotNet(ModelType.CNN_2D, ref.random_weights(ref.CNN_2D), device=0)
+    """In a child process that sees no device (CUDA_VISIBLE_DEVICES empty), so that a machine with a GPU checks this too."""
+    import os
+    import subprocess
+    import sys
+
+    from tests.conftest import ROOT
+    code = ("import pytest\nfrom oracle import pilot_ref as ref\nfrom triton_racer_sim_b200 import _native as nat\n"
+            "from triton_racer_sim_b200.pilot import ModelType, PilotNet\n"
+            "with pytest.raises((nat.NativeError, RuntimeError)):\n    PilotNet(ModelType.CNN_2D, ref.random_weights(ref.CNN_2D), device=0)\n")
+    run = subprocess.run([sys.executable, "-c", code], cwd=ROOT, env=dict(os.environ, CUDA_VISIBLE_DEVICES=""), capture_output=True, text=True,
+                         timeout=300)
+    assert run.returncode == 0, run.stderr[-2000:]
 
 
 # ---- the reference's own model-building and step code, executed over a numpy stand-in for the Keras primitives (tests/golden/pilot.npz) ----------
