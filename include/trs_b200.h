@@ -213,6 +213,23 @@ int trs_telemetry_decode_host(trs_ctx* ctx, const char* text_host, const unsigne
                               uint8_t* out_u8_dev, void* stream);
 
 /*
+ * Tub recording: batched JPEG encode of N device frames, replacing
+ *   Image.fromarray(img).save(path)      TritonRacerSim/components/datastorage.py:78 (the recorder's cam/processed_img, manage.py:103-104)
+ *   cv2.imwrite(path, img)               TritonRacerSim/utils/post_process.py (the same bytes at the same quality)
+ * Baseline JPEG, YCbCr 4:2:0, libjpeg quality scaling, standard Huffman tables: byte-identical with Pillow / libjpeg(-turbo)
+ * (Pillow's default quality is 75, OpenCV's 95).
+ *   frames_dev    (N, h, w, 3) uint8 RGB on the device, h and w in 1..65535; quality in 1..100
+ *   offsets_host  receives N + 1 byte offsets of the packed files (file k = [offsets[k], offsets[k+1]))
+ * Encodes into the context's staging (grown when a call needs more): a counting pass gives the exact size of every file, `stream`
+ * is synchronised, the offsets are written, and the files are written back to back behind their offsets on `stream`.
+ */
+int trs_jpeg_encode(trs_ctx* ctx, const uint8_t* frames_dev, int n, int h, int w, int quality, unsigned long long* offsets_host,
+                    void* stream);
+/* Copies the packed files of the last trs_jpeg_encode on this context (bytes must equal its offsets_host[n]) to blob_host
+ * (pageable or pinned); call it on the stream of that encode.  Synchronises `stream`.  TRS_E_STATE: no encode yet. */
+int trs_jpeg_encode_copy(trs_ctx* ctx, uint8_t* blob_host, unsigned long long bytes, void* stream);
+
+/*
  * Forward pass of the pilots' networks (SURVEY.md 8(f) rank 4), replacing for N frames
  *   self.model(img_arr) / self.model((img_arr, spd)) / self.model((img_arr, spd, features))
  *                                           TritonRacerSim/components/keras_pilot.py:59,71,81,104

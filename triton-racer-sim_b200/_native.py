@@ -19,7 +19,7 @@ SYMBOLS = [
     "trs_version", "trs_last_error", "trs_kernel_launches", "trs_ctx_create", "trs_ctx_destroy", "trs_ctx_device_info",
     "trs_set_preproc_params", "trs_preprocess", "trs_normalise", "trs_set_track", "trs_locate", "trs_speed_control",
     "trs_preprocess_host", "trs_host_alloc", "trs_host_free", "trs_debug_canny_stages", "trs_control_mux", "trs_pwm_map",
-    "trs_jpeg_decode_host", "trs_telemetry_decode_host",
+    "trs_jpeg_decode_host", "trs_telemetry_decode_host", "trs_jpeg_encode", "trs_jpeg_encode_copy",
     "trs_pilot_create", "trs_pilot_destroy", "trs_pilot_forward", "trs_pilot_debug_activation", "trs_pilot_layer_shape",
     "trs_pilot_cap", "trs_probe_fp64",
 ]
@@ -97,6 +97,8 @@ def load():
     lib.trs_pwm_map.argtypes = [vp, vp, i32, C.c_double, C.c_double, C.c_double, vp, vp]
     lib.trs_jpeg_decode_host.argtypes = [vp, vp, vp, i32, i32, i32, vp, vp]
     lib.trs_telemetry_decode_host.argtypes = [vp, vp, vp, i32, i32, i32, vp, vp]
+    lib.trs_jpeg_encode.argtypes = [vp, vp, i32, i32, i32, i32, vp, vp]
+    lib.trs_jpeg_encode_copy.argtypes = [vp, vp, C.c_ulonglong, vp]
     lib.trs_pilot_create.argtypes = [vp, i32, i32, i32, C.POINTER(Tensor), i32, i32, C.POINTER(vp)]
     lib.trs_pilot_destroy.argtypes = [vp]
     lib.trs_pilot_forward.argtypes = [vp, vp, i32, vp, vp, vp, vp]

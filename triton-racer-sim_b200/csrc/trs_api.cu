@@ -22,6 +22,7 @@
 #include "../../include/trs_b200.h"
 #include "jpeg_host.h"
 #include "jpeg_kernels.cuh"
+#include "jpeg_enc_kernels.cuh"
 #include "misc_kernels.cuh"
 #include "preproc_kernel.cuh"
 #include "preproc_fast.cuh"
@@ -105,6 +106,13 @@ struct trs_ctx {
     uint8_t* jpg_blob = nullptr;   size_t jpg_blob_cap = 0;
     uint8_t* jpg_planes = nullptr; size_t jpg_planes_cap = 0;
     void* jpg_meta = nullptr;      size_t jpg_meta_cap = 0;
+    // tub recording (trs_jpeg_encode): tables + header of the last (h, w, quality), per-record sizes / offsets, the packed files
+    uint8_t* jpe_meta = nullptr;   int jpe_meta_key[3] = {0, 0, 0};
+    unsigned long long* jpe_sizes = nullptr; size_t jpe_sizes_cap = 0;         // records; the offsets buffer holds one more
+    unsigned long long* jpe_offs = nullptr;
+    uint8_t* jpe_blob = nullptr;   size_t jpe_blob_cap = 0;
+    long long jpe_last_bytes = -1;                                             // bytes of the last encode, -1: none yet
+    std::vector<unsigned long long> jpe_host_offs;
 };
 
 int trs_i_fail(int code, const char* fmt, ...)
@@ -502,6 +510,7 @@ int trs_ctx_destroy(trs_ctx* ctx)
     cudaFree(ctx->wp_dev); cudaFree(ctx->wp_grid_dev); cudaFree(ctx->wp_cells_dev); cudaFree(ctx->defer_dev);
     cudaFree(ctx->stats_dev);
     cudaFree(ctx->jpg_blob); cudaFree(ctx->jpg_planes); cudaFree(ctx->jpg_meta);
+    cudaFree(ctx->jpe_meta); cudaFree(ctx->jpe_sizes); cudaFree(ctx->jpe_offs); cudaFree(ctx->jpe_blob);
     delete ctx;
     return 0;
 }
@@ -899,6 +908,90 @@ int trs_jpeg_decode_host(trs_ctx* ctx, const uint8_t* blob_host, const unsigned 
     CU(cudaMemcpyAsync(&status, d_status, sizeof(int), cudaMemcpyDeviceToHost, st));
     CU(cudaStreamSynchronize(st));                              // recs / sets (host vectors) and the staging buffers are reused
     if (status) return fail(TRS_E_RANGE, "corrupt entropy-coded data in at least one record (decoder status %d)", status);
+    return 0;
+}
+
+int trs_jpeg_encode(trs_ctx* ctx, const uint8_t* frames_dev, int n, int h, int w, int quality, unsigned long long* offsets_host,
+                    void* stream)
+{
+    TRS_ENTER(ctx);
+    if (n < 0) return fail(TRS_E_ARG, "negative record count %d", n);
+    if (h < 1 || h > 65535 || w < 1 || w > 65535) return fail(TRS_E_ARG, "frame size %dx%d outside 1..65535", h, w);
+    if (quality < 1 || quality > 100) return fail(TRS_E_ARG, "quality %d outside 1..100", quality);
+    if (!offsets_host) return fail(TRS_E_ARG, "null offsets_host");
+    if (n > 0 && !frames_dev) return fail(TRS_E_ARG, "null frames_dev");
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    ctx->jpe_last_bytes = -1;
+    offsets_host[0] = 0;
+    if (n == 0) { ctx->jpe_last_bytes = 0; return 0; }
+    cudaStream_t st = (cudaStream_t)stream;
+    // tables and headers depend only on (h, w, quality): built on the host, uploaded when they change
+    const size_t meta_bytes = sizeof(trs::JpeEncTables) + trs::JPE_HEADER_BYTES;
+    if (!ctx->jpe_meta) { CU(cudaMalloc(&ctx->jpe_meta, meta_bytes)); ctx->jpe_meta_key[0] = 0; }
+    if (ctx->jpe_meta_key[0] != h || ctx->jpe_meta_key[1] != w || ctx->jpe_meta_key[2] != quality) {
+        std::vector<uint8_t> meta(meta_bytes);
+        trs::JpeEncTables T;
+        trs::jpe_make_tables(quality, T);
+        memcpy(meta.data(), &T, sizeof T);
+        trs::jpe_build_header(h, w, quality, meta.data() + sizeof T);
+        ctx->jpe_meta_key[0] = 0;
+        CU(cudaMemcpyAsync(ctx->jpe_meta, meta.data(), meta_bytes, cudaMemcpyHostToDevice, st));
+        CU(cudaStreamSynchronize(st));                                              // `meta` is a local vector
+        ctx->jpe_meta_key[0] = h; ctx->jpe_meta_key[1] = w; ctx->jpe_meta_key[2] = quality;
+    }
+    const trs::JpeEncTables* d_tables = reinterpret_cast<const trs::JpeEncTables*>(ctx->jpe_meta);
+    const uint8_t* d_header = ctx->jpe_meta + sizeof(trs::JpeEncTables);
+    if (ctx->jpe_sizes_cap < (size_t)n) {
+        cudaFree(ctx->jpe_sizes); cudaFree(ctx->jpe_offs);
+        ctx->jpe_sizes = ctx->jpe_offs = nullptr; ctx->jpe_sizes_cap = 0;
+        CU(cudaMalloc(&ctx->jpe_sizes, (size_t)n * sizeof(unsigned long long)));
+        CU(cudaMalloc(&ctx->jpe_offs, ((size_t)n + 1) * sizeof(unsigned long long)));
+        ctx->jpe_sizes_cap = (size_t)n;
+    }
+    const int smem = (int)sizeof(trs::JpeSmem);
+    CU(cudaFuncSetAttribute(trs::k_jpeg_encode<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    CU(cudaFuncSetAttribute(trs::k_jpeg_encode<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
+    int per_sm = 0;
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, trs::k_jpeg_encode<true>, trs::JPE_THREADS, smem));
+    if (per_sm < 1) return fail(TRS_E_RANGE, "encoder does not fit an SM with %d B shared memory", smem);
+    const int grid = n < ctx->sm_count * per_sm ? n : ctx->sm_count * per_sm;
+    // pass 1: exact file sizes (the same arithmetic as pass 2, nothing written but the sizes)
+    trs::k_jpeg_encode<false><<<grid, trs::JPE_THREADS, smem, st>>>(frames_dev, n, h, w, d_tables, d_header, ctx->jpe_sizes, nullptr, nullptr);
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    CU(cudaGetLastError());
+    std::vector<unsigned long long>& offs = ctx->jpe_host_offs;
+    offs.assign((size_t)n + 1, 0);
+    CU(cudaMemcpyAsync(offs.data() + 1, ctx->jpe_sizes, (size_t)n * sizeof(unsigned long long), cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
+    for (size_t k = 1; k <= (size_t)n; ++k) offs[k] += offs[k - 1];
+    const size_t total = (size_t)offs[(size_t)n];
+    if (ctx->jpe_blob_cap < total) {
+        cudaFree(ctx->jpe_blob); ctx->jpe_blob = nullptr; ctx->jpe_blob_cap = 0;
+        CU(cudaMalloc(&ctx->jpe_blob, total));
+        ctx->jpe_blob_cap = total;
+    }
+    // pass 2: every file at its offset
+    CU(cudaMemcpyAsync(ctx->jpe_offs, offs.data(), ((size_t)n + 1) * sizeof(unsigned long long), cudaMemcpyHostToDevice, st));
+    trs::k_jpeg_encode<true><<<grid, trs::JPE_THREADS, smem, st>>>(frames_dev, n, h, w, d_tables, d_header, nullptr, ctx->jpe_offs, ctx->jpe_blob);
+    g_launches.fetch_add(1, std::memory_order_relaxed);
+    CU(cudaGetLastError());
+    memcpy(offsets_host, offs.data(), ((size_t)n + 1) * sizeof(unsigned long long));
+    ctx->jpe_last_bytes = (long long)total;
+    return 0;
+}
+
+int trs_jpeg_encode_copy(trs_ctx* ctx, uint8_t* blob_host, unsigned long long bytes, void* stream)
+{
+    TRS_ENTER(ctx);
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    if (ctx->jpe_last_bytes < 0) return fail(TRS_E_STATE, "no successful trs_jpeg_encode on this context");
+    if (bytes != (unsigned long long)ctx->jpe_last_bytes)
+        return fail(TRS_E_ARG, "bytes = %llu, but the last trs_jpeg_encode produced %lld", bytes, ctx->jpe_last_bytes);
+    if (bytes == 0) return 0;
+    if (!blob_host) return fail(TRS_E_ARG, "null blob_host");
+    cudaStream_t st = (cudaStream_t)stream;
+    CU(cudaMemcpyAsync(blob_host, ctx->jpe_blob, (size_t)bytes, cudaMemcpyDeviceToHost, st));
+    CU(cudaStreamSynchronize(st));
     return 0;
 }
 

@@ -5,6 +5,8 @@ The reference's trainers read a tub folder record by record (components/keras_tr
 ``json.load``; the recorder writes them with ``Image.fromarray(img).save(path)`` (components/datastorage.py:67-79).  Here the JPEG
 files of a batch are decoded by the CUDA kernels behind ``trs_jpeg_decode_host`` straight into the ``(N,H,W,3)`` uint8 device tensor
 the rest of the path reads (bit-exact with Pillow's decoder), so only the ~5 KB files cross the PCIe link, not 57.6 KB of pixels.
+The write side is the same trade in the other direction: ``encode_jpeg_batch`` / ``TubWriter`` encode device frames behind
+``trs_jpeg_encode`` (byte-identical with Pillow's ``save``) and only the files come back to the host.
 """
 from __future__ import annotations
 
@@ -69,6 +71,79 @@ def decode_jpeg_batch(files, hw=None, device=None, ctx=None, out=None) -> torch.
         if own:
             ctx.close()
     return out
+
+
+def encode_jpeg_batch(frames: torch.Tensor, quality: int = 75, device=None, ctx=None):
+    """Encode a CUDA uint8 (N,H,W,3) RGB tensor into N baseline-JPEG files, byte-identical with
+    ``Image.fromarray(frame).save(f, "JPEG", quality=quality)`` (the recorder's call, datastorage.py:78; Pillow's default quality is 75,
+    ``cv2.imencode``'s 95).  Returns ``(blob uint8 array, offsets uint64 array of N + 1 entries)``, the form ``decode_jpeg_batch``
+    takes.  The encoding runs on the frames' stream-ordered position on the current stream; only the files are copied back."""
+    if not isinstance(frames, torch.Tensor) or not frames.is_cuda:
+        raise TypeError("frames must be a CUDA tensor")
+    if frames.dtype != torch.uint8 or frames.dim() != 4 or frames.shape[3] != 3:
+        raise ValueError(f"frames must be uint8 (N,H,W,3), got {tuple(frames.shape)} {frames.dtype}")
+    if not frames.is_contiguous():
+        raise ValueError("frames must be contiguous")
+    quality = int(quality)
+    n, h, w = int(frames.shape[0]), int(frames.shape[1]), int(frames.shape[2])
+    own = ctx is None
+    dev = frames.device.index if device is None else int(device if not isinstance(device, torch.device) else device.index)
+    if dev != frames.device.index:
+        raise ValueError(f"frames are on cuda:{frames.device.index}, the encoder runs on cuda:{dev}")
+    ctx = nat.Context(dev) if own else ctx
+    try:
+        if ctx.device != frames.device.index:
+            raise ValueError(f"frames are on cuda:{frames.device.index}, the context on cuda:{ctx.device}")
+        offsets = np.zeros(n + 1, np.uint64)
+        stream = C.c_void_p(torch.cuda.current_stream(ctx.device).cuda_stream)
+        nat.check(ctx.lib.trs_jpeg_encode(ctx.handle, C.c_void_p(frames.data_ptr() if n else 0), n, h, w, quality,
+                                          C.c_void_p(offsets.ctypes.data), stream), "trs_jpeg_encode")
+        blob = np.empty(int(offsets[n]), np.uint8)
+        nat.check(ctx.lib.trs_jpeg_encode_copy(ctx.handle, C.c_void_p(blob.ctypes.data if blob.size else 0), C.c_ulonglong(blob.size), stream),
+                  "trs_jpeg_encode_copy")
+    finally:
+        if own:
+            ctx.close()
+    return blob, offsets
+
+
+class TubWriter:
+    """The write side of ``TubReader``: a batch of records in the layout and numbering of the reference's recorder
+    (components/datastorage.py:67-79, :98-112): ``img_{i}.jpg`` + ``record_{i}.json`` with ``'cam/img'`` holding the file name,
+    numbered from 0 (the loaders read from 1, ``count_records``).  The frames are encoded on the GPU (``encode_jpeg_batch``), the
+    files and JSON records are written by the host.  The recorder's thread, toggle and delete handling are not part of this."""
+
+    def __init__(self, tub_path: str, device=None, quality: int = 75):
+        self.path = tub_path
+        self.device = torch.cuda.current_device() if device is None else int(device)
+        self.quality = int(quality)
+        self.index = 0                                   # next record number (datastorage.py: the file thread counts from 0)
+        self.ctx = nat.Context(self.device)
+        os.makedirs(tub_path, exist_ok=True)
+
+    def write(self, frames: torch.Tensor, records):
+        """frames: CUDA uint8 (N,H,W,3) (the recorder's ``cam/img`` input); records: N dicts of the other values.  Returns the record
+        numbers written."""
+        records = list(records)
+        if len(records) != int(frames.shape[0]):
+            raise ValueError(f"{int(frames.shape[0])} frames but {len(records)} records")
+        blob, offsets = encode_jpeg_batch(frames, self.quality, device=self.device, ctx=self.ctx)
+        written = []
+        for k, rec in enumerate(records):
+            i = self.index + k
+            name = f"img_{i}.jpg"
+            with open(os.path.join(self.path, name), "wb") as f:
+                f.write(blob[int(offsets[k]):int(offsets[k + 1])].tobytes())
+            row = {"cam/img": name}
+            row.update({key: v for key, v in rec.items() if key != "cam/img"})
+            with open(os.path.join(self.path, f"record_{i}.json"), "w") as f:
+                json.dump(row, f)
+            written.append(i)
+        self.index += len(records)
+        return written
+
+    def close(self):
+        self.ctx.close()
 
 
 # The reference's loader classes differ only in what they take from a record (keras_train.py:113-119, 264-299):
