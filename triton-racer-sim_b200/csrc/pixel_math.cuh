@@ -61,6 +61,15 @@ TRS_HD uint32_t sat_threshold_entry(long long K, int v, int sd)
     return (uint32_t)(q < v ? q : v);
 }
 
+// ... with the value bounds [vlo, vhi] of the same range folded in (the table is indexed by v already): a value outside them gets a threshold no
+// delta passes, 0x8001 (-1) for an upper saturation bound "d <= T" and 255 for a lower one "d > T" (d <= v <= 255).  `upper`: which of the two the
+// entry serves; K as for sat_threshold_entry.
+TRS_HD uint32_t sat_threshold_entry_folded(long long K, bool upper, int v, int sd, long long vlo, long long vhi)
+{
+    if (v < vlo || v > vhi) return upper ? 0x8001u : 255u;
+    return sat_threshold_entry(K, v, sd);
+}
+
 // Hue bounds without computing the hue (preproc_fast.cuh, HueThresholds): h = (h0 hdiv[d] + 2048) >> 12 is monotone in the numerator h0, and a
 // wrapped hue (h0 < 0: h + 180 >= 150) cannot pass an upper bound <= 149, so "lo <= h <= hi" is "a_lo <= h0 <= a_hi" for such a bound: the smallest
 // numerator with h0 hd + 2048 >= 4096 lo and the largest with h0 hd + 2048 <= 4096 hi + 4095.  Returned biased by 2048 like the packed numerators, as

@@ -274,6 +274,15 @@ __device__ __forceinline__ uint32_t hge_mask(uint32_t a, uint32_t b) { return __
 __device__ __forceinline__ uint32_t hle_mask(uint32_t a, uint32_t b) { return __hle2_mask(h2(a), h2(b)); }
 __device__ __forceinline__ uint32_t heq_mask(uint32_t a, uint32_t b) { return __heq2_mask(h2(a), h2(b)); }
 __device__ __forceinline__ uint32_t bsel(uint32_t m, uint32_t a, uint32_t b) { return (a & m) | (b & ~m); }                      // one LOP3
+// (a0, a1) * b + (c0, c1) as ONE packed fp32 instruction (fma.rn.f32x2, SASS FFMA2: |x| / -x operand modifiers fold as for FFMA); each lane is a
+// correctly rounded fma, bit-identical with __fmaf_rn.  Returns the two results' bit patterns.
+__device__ __forceinline__ uint2 ffma2_bits(float a0, float a1, float b, float c0, float c1)
+{
+    uint2 d;
+    asm("{\n.reg .b64 a, b, c, d;\nmov.b64 a, {%2, %3};\nmov.b64 b, {%4, %4};\nmov.b64 c, {%5, %6};\nfma.rn.f32x2 d, a, b, c;\nmov.b64 {%0, %1}, d;\n}\n"
+        : "=r"(d.x), "=r"(d.y) : "f"(a0), "f"(a1), "f"(b), "f"(c0), "f"(c1));
+    return d;
+}
 
 // direction class (pixel_math.cuh canny_dir) from sign bits: horizontal <=> ay*2^15 - ax*13573 < 0,
 // vertical <=> ax*79109 - ay*2^15 < 0, else diagonal 2 + (sign(dx) != sign(dy))
@@ -380,10 +389,13 @@ __device__ __forceinline__ uint32_t live_flags(const FastRange& R) { return F >=
 // compile-time constants with at most two saturation bounds, the 256-entry table (in the place of sdiv) holds the two thresholds of a
 // value v as 16-bit halves: one table read per pixel, two packed compares per pixel pair, no multiply / shift / repack.
 // Bounds take table halves in range order, the lower bound of a range before its upper bound.
+// A range with a saturation bound in the table also has its value bounds folded into its thresholds (sat_threshold_entry_folded: a value outside
+// them gets a threshold no delta passes), so its value compares are not emitted; a range without one keeps them.
 template <int NR, int F0, int F1>
 struct SatThresholds {
     static constexpr int n = (F0 >= 0 && F1 >= 0 && NR == 2) ? ((F0 >> 2) & 1) + ((F0 >> 3) & 1) + ((F1 >> 2) & 1) + ((F1 >> 3) & 1) : 99;
     static constexpr bool use = n >= 1 && n <= 2;
+    __host__ __device__ static constexpr bool folds(int r) { return use && (((r == 0 ? F0 : F1) & 12) != 0); }
 };
 
 // Hue bounds without computing the hue: h = (h0 * hdiv[d] + 2048) >> 12 is monotone in the numerator h0, and the wrapped values (h0 < 0:
@@ -451,8 +463,10 @@ __device__ __forceinline__ void hsv_masks_of(const FastParams& P, const uint32_t
                 if (fl[r] & 4u) ok &= hge_mask(s2, R.lo[1]);
                 if (fl[r] & 8u) ok &= hle_mask(s2, R.hi[1]);
             }
-            if (fl[r] & 16u) ok &= hge_mask(v2[half], R.lo[2]);
-            if (fl[r] & 32u) ok &= hle_mask(v2[half], R.hi[2]);
+            if (!SatThresholds<NR, F0, F1>::folds(r)) {
+                if (fl[r] & 16u) ok &= hge_mask(v2[half], R.lo[2]);
+                if (fl[r] & 32u) ok &= hle_mask(v2[half], R.hi[2]);
+            }
             okm[r][half] = ok;
             if (hl[r]) alive |= ok;
         }
@@ -619,7 +633,8 @@ __device__ __forceinline__ void p1_strip_walk(const FastParams& P, const Dims& D
             // direction class of each pixel pair, branch-free, mostly on the FMA pipe (pixel_math.cuh canny_dir):
             //   horizontal <=> |dy| - |dx| 13573/2^15 < 0,  vertical <=> |dx| 79109/2^15 - |dy| < 0,  else diagonal 2 + (sign dx != sign dy)
             // the halves are widened to fp32 (exact: n * 2^-24) and each test is ONE fused multiply-add whose sign is exact
-            // (the rounding of an fma never changes the sign of a non-zero exact result and an exact zero stays +0)
+            // (the rounding of an fma never changes the sign of a non-zero exact result and an exact zero stays +0); the two pixels of a pair
+            // share one packed FFMA2 per test
             uint32_t code[2];
 #pragma unroll
             for (int half = 0; half < 2; ++half) {
@@ -627,9 +642,9 @@ __device__ __forceinline__ void p1_strip_walk(const FastParams& P, const Dims& D
                 const float ax_lo = fabsf(__low2float(hx)), ax_hi = fabsf(__high2float(hx));
                 const float ay_lo = fabsf(__low2float(hy)), ay_hi = fabsf(__high2float(hy));
                 const float T22 = 13573.0f / 32768.0f, T67 = 79109.0f / 32768.0f;      // both exact in fp32 (14- and 17-bit numerators)
-                const uint32_t nu_lo = __float_as_uint(__fmaf_rn(ax_lo, -T22, ay_lo)), nu_hi = __float_as_uint(__fmaf_rn(ax_hi, -T22, ay_hi));
-                const uint32_t wv_lo = __float_as_uint(__fmaf_rn(ax_lo, T67, -ay_lo)), wv_hi = __float_as_uint(__fmaf_rn(ax_hi, T67, -ay_hi));
-                const uint32_t H2 = prmt_sx(nu_lo, nu_hi, 0xffbb), V2 = prmt_sx(wv_lo, wv_hi, 0xffbb);       // sign of each result spread over its half
+                const uint2 nu = ffma2_bits(ax_lo, ax_hi, -T22, ay_lo, ay_hi);
+                const uint2 wv = ffma2_bits(ax_lo, ax_hi, T67, -ay_lo, -ay_hi);
+                const uint32_t H2 = prmt_sx(nu.x, nu.y, 0xffbb), V2 = prmt_sx(wv.x, wv.y, 0xffbb);       // sign of each result spread over its half
                 const uint32_t SD = prmt_sx(dxs[half] ^ dys[half], 0, 0xbb99);
                 const uint32_t diag = (SD & 0x00010001u) | 0x00020002u;
                 code[half] = ~H2 & bsel(V2, 0x00010001u, diag);
@@ -1050,7 +1065,8 @@ __device__ __forceinline__ void init_tables(const PreKParams& p, const SmemMap& 
     for (int i = t0; i < 256; i += tstride) {
         const int sd = hsv_sdiv_entry(i);
         if (SatThresholds<NR, F0, F1>::use) {
-            // the live saturation bounds in table order (see SatThresholds); K = the largest admissible saturation of "s <= K"
+            // the live saturation bounds in table order (see SatThresholds); K = the largest admissible saturation of "s <= K"; the range's
+            // value bounds folded in
             uint32_t entry = 0;
             int slot = 0;
 #pragma unroll
@@ -1060,7 +1076,7 @@ __device__ __forceinline__ void init_tables(const PreKParams& p, const SmemMap& 
                 for (int side = 0; side < 2; ++side) {
                     if (!(fl & (4 << side))) continue;
                     const long long K = side == 0 ? (long long)p.ranges[r].lo[1] - 1 : (long long)p.ranges[r].hi[1];
-                    entry |= sat_threshold_entry(K, i, sd) << (16 * (slot & 1));
+                    entry |= sat_threshold_entry_folded(K, side == 1, i, sd, p.ranges[r].lo[2], p.ranges[r].hi[2]) << (16 * (slot & 1));
                     ++slot;
                 }
             }
