@@ -71,7 +71,8 @@ typedef struct trs_spd_params {
 /* Per-call statistics written by trs_preprocess (all counters are sums over the N frames). */
 enum {
     TRS_STAT_FRAMES = 0,     /* frames processed                                   */
-    TRS_STAT_MASK0 = 1,      /* set pixels of colour range 0..3                    */
+    TRS_STAT_MASK0 = 1,      /* set pixels of colour range 0..3; 0 for a range whose channel a later range or the edge
+                                layer overwrites (trs_set_preproc_params drops it, it never reaches the output)        */
     TRS_STAT_MASK1 = 2,
     TRS_STAT_MASK2 = 3,
     TRS_STAT_MASK3 = 4,

@@ -63,14 +63,15 @@ def reduction_len(layer):
 
 # ---- fp64 evaluation on the kernels' operands ----------------------------------------------------------------------------------
 
-def conv_exact(x_nhwc, kern16, stride):
+def conv_exact(x_nhwc, kern16, stride, device="cpu"):
     """S and A of a VALID convolution, NHWC float64.  x: the layer's input as the kernel sees it (u8 bytes for conv1, the fp16
     activation otherwise); kern16: (kh, kw, Cin, Cout) fp16.  fp16 x fp16 and u8 x fp16 products are exact in fp64; the fp64 sums
-    are within ~K * 2^-53 * A of the exact ones, 2^-25 below the smallest E_acc."""
-    x = torch.from_numpy(np.asarray(x_nhwc).astype(np.float64)).permute(0, 3, 1, 2)
-    k = torch.from_numpy(np.asarray(kern16).astype(np.float64)).permute(3, 2, 0, 1).contiguous()
-    s = F.conv2d(x, k, stride=stride).permute(0, 2, 3, 1).numpy()
-    a = F.conv2d(x.abs(), k.abs(), stride=stride).permute(0, 2, 3, 1).numpy()
+    are within ~K * 2^-53 * A of the exact ones in any summation order, 2^-25 below the smallest E_acc, so `device` may be a GPU
+    (float64 convolutions there sum in another order than on the CPU)."""
+    x = torch.from_numpy(np.asarray(x_nhwc).astype(np.float64)).to(device).permute(0, 3, 1, 2)
+    k = torch.from_numpy(np.asarray(kern16).astype(np.float64)).to(device).permute(3, 2, 0, 1).contiguous()
+    s = F.conv2d(x, k, stride=stride).permute(0, 2, 3, 1).cpu().numpy()
+    a = F.conv2d(x.abs(), k.abs(), stride=stride).permute(0, 2, 3, 1).cpu().numpy()
     return s, a
 
 
@@ -166,9 +167,9 @@ def layer_kernels(h, w, rowconv=True, frames_16_aligned=True, full_house=False):
     return out
 
 
-def worst(report, box, count=6):
+def worst(report, box, count=6, frame0=0):
     """The `count` largest err / bound elements of an (N, H, W, C) report: (frame, y, x, channel), their position in the layer's box
-    (bx, by, bn), err, bound and the exact value."""
+    (bx, by, bn), err, bound and the exact value.  frame0: the batch index of the report's first frame."""
     r = report["ratio"]
     bx, by, bn = box
     exact = report.get("yhat")
@@ -176,6 +177,7 @@ def worst(report, box, count=6):
     for f in np.argsort(r, axis=None)[::-1][:count]:
         i = np.unravel_index(f, r.shape)
         n, yy, xx, c = i
+        n += frame0
         lines.append(f"(n={n}, y={yy}, x={xx}, c={c}) in box (n%{bn}={n % bn}, y%{by}={yy % by}, x%{bx}={xx % bx}): "
                      f"err/bound={r[i]:.3g} err={report['err'][i]:.4g} bound={report['bound'][i]:.4g}"
                      + (f" exact={exact[i]:.6g}" if exact is not None else ""))

@@ -170,18 +170,81 @@ def test_bad_arguments_raise():
         LocationTracker('/nonexistent/track.json', device=0)
 
 
-def test_statistics_match_oracle_counts():
-    cfg = full_house_config()
-    frames = synth.frame_pool(64, 120, 160, seed=5)
-    want = oracle.process_batch(frames, cfg)
-    comp = ImgPreprocessing(cfg, device=0, collect_stats=True)
-    comp.process_device(torch.from_numpy(frames).to(DEV))
-    st = comp.stats()
-    assert st["frames"] == 64
-    assert st["mask0"] == int((want[..., 0] == 255).sum())
-    assert st["mask1"] == int((want[..., 1] == 255).sum())
-    assert st["edge"] == int((want[..., 2] == 255).sum())
-    comp.onShutdown()
+def oracle_counts(frames, cfg, want):
+    """The counters trs_preprocess must report for `frames` (TRS_STAT_*), from the oracle.  A colour range whose output channel a
+    later range or the edge layer overwrites never reaches the output and counts 0; strong / cand count the NMS map's 2s and
+    non-zeros, taken on the frame after its brightness / contrast table; the ROI sum covers rows 40..118 when the table is dynamic."""
+    p = oracle.params_from_cfg(cfg)
+    c = dict(frames=len(frames), mask0=0, mask1=0, mask2=0, mask3=0, edge=0, strong=0, cand=0, roi_sum=0)
+    layers = [(f"mask{i}", p.color_dest[i] % 3) for i in range(p.n_hsv if p.color_filter_enabled else 0)]
+    layers += [("edge", p.edge_dest % 3)] if p.edge_enabled else []
+    for k, (name, ch) in enumerate(layers):
+        if all(later != ch for _, later in layers[k + 1:]):
+            c[name] = int((want[..., ch] == 255).sum())
+    if p.edge_enabled:
+        for img in frames:
+            lut, _ = oracle.brightness_lut(img, cfg)
+            _, _, mp = oracle.canny3(lut[img], p.canny_a, p.canny_b, taps=True)
+            c["strong"] += int((mp == 2).sum())
+            c["cand"] += int((mp >= 1).sum())
+    if p.dynamic_brightness:
+        c["roi_sum"] = int(frames[:, 40:119].astype(np.uint64).sum())
+    return c
+
+
+# (switch, h, w, configuration, frames, CTAs per SM at most): every kernel launch_preprocess picks (trs_api.cu:302-437), with at least
+# five frames per CTA.  The grid is SMs x CTAs per SM: two for the resident / banded / store-warp kernels (trs_api.cu:374) and for
+# k_preprocess_bsw (384 threads at <= 80 registers: 65,536 registers hold two), eight for k_adjust_stream (trs_api.cu:308), and at most
+# 2,048 / 512 threads = four for the generic kernel (trs_api.cu:432).
+STAT_KERNELS = {
+    "store_warp_120x160": (None, 120, 160, "full_house", 1500, 2),
+    "banded_store_warp_240x320": (None, 240, 320, "full_house", 1500, 2),
+    "resident_no_store_warp": ("TRS_NO_STORE_WARP", 120, 160, "full_house", 1500, 2),
+    "banded_no_store_warp": ("TRS_NO_STORE_WARP", 240, 320, "full_house", 1500, 2),
+    "table_dyn_contrast": (None, 120, 160, "dyn_contrast", 1500, 2),
+    "table_exotic": (None, 120, 160, "exotic", 1500, 2),
+    "no_filter_adjust_stream": (None, 120, 160, "adjust_dynamic", 5920, 8),
+    "generic_122x166": ("TRS_FORCE_GENERIC", 122, 166, "full_house", 2960, 4),
+    "generic_7x9": (None, 7, 9, "exotic", 2960, 4),
+}
+
+
+@pytest.mark.timeout(600)
+def test_statistics_match_oracle_counts(golden_images, monkeypatch):
+    """Every counter but the sweeps and the timers against the oracle, for every kernel: the kernels count strong and candidate
+    pixels in different places (before the hysteresis in the banded store-warp kernel, from the finished planes in the store
+    warps, in the suppression loop of the generic kernel).  All kernels are checked before the test fails, and the message names
+    each one that disagrees."""
+    from tests.helpers import image_cases
+    ctx = nat.Context(0)
+    sms = ctx.sm_count
+    ctx.close()
+    cases = image_cases(golden_images)
+    extra = dict(adjust_dynamic=dict(preprocessing_dynamic_brightness_enabled=True, preprocessing_contrast_enhancement_ratio=1.25,
+                                     preprocessing_brightness_baseline=380))
+    failures = []
+    for name, (env, h, w, cname, n, per_sm) in STAT_KERNELS.items():
+        assert n >= 5 * sms * per_sm, f"{name}: {n} frames on up to {sms * per_sm} CTAs is fewer than five frames per CTA"
+        for switch in ("TRS_NO_STORE_WARP", "TRS_FORCE_GENERIC"):
+            monkeypatch.delenv(switch, raising=False)
+        if env:
+            monkeypatch.setenv(env, "1")                     # read when the component's context is created
+        cfg = cfg_for(cases[cname] if cname in cases else extra[cname])
+        frames = synth.expand_numpy(synth.frame_pool(64, h, w, seed=5), n, start=11)
+        want = oracle.process_batch(frames, cfg)
+        comp = ImgPreprocessing(cfg, device=0, collect_stats=True)
+        got, _ = comp.process_device(torch.from_numpy(frames).to(DEV), want_f32=False)
+        st = comp.stats()
+        comp.onShutdown()
+        got = got.cpu().numpy()
+        if not np.array_equal(got, want):
+            failures.append(f"{name}: output {describe(got, want)}")
+            continue
+        want_st = oracle_counts(frames, cfg, want)
+        bad = [f"{k} {st[k]} != {v}" for k, v in want_st.items() if st[k] != v]
+        if bad:
+            failures.append(f"{name}: " + ", ".join(bad))
+    assert not failures, "\n".join(failures)
 
 
 def test_normalise_and_crop_resize():
