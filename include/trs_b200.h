@@ -142,6 +142,26 @@ int trs_locate(trs_ctx* ctx, const double* xyz_dev, int n, int32_t* idx_dev, dou
                void* stream);
 
 /*
+ * Several centre lines in one batch: what one LocationTracker per car does when the cars come from simulators on different
+ * tracks (every car builds its own, manage.py:97-99).  Independent of trs_set_track / trs_locate: a context can hold both.
+ * Upload n_tracks centre lines (host pointers wp_xyz_host[t], n_wp[t] x 3 f64) with their segment ranges min_map[t], max_map[t];
+ * 1 <= n_tracks <= TRS_MAX_TRACKS, every n_wp[t] > 0.  Replaces the previous set.
+ */
+#define TRS_MAX_TRACKS 256
+int trs_set_tracks(trs_ctx* ctx, const double* const* wp_xyz_host, const int* n_wp, const double* min_map,
+                   const double* max_map, int n_tracks);
+
+/*
+ * Nearest waypoint of N cars, car i on track track_dev[i]: exactly what trs_locate returns for it with that track alone.
+ *   xyz_dev (N,3) f64; track_dev (N) i32; idx_dev (N) i32 — nullable; segment_dev (N) f64 — nullable.
+ *   A track index outside [0, n_tracks) gives idx -1 and segment NaN (nothing is reported to the host: the call does not synchronise).
+ *   No allocation after the first call of a given N.  Large batches keep per-context scratch (bucketed cars, the list of cars
+ *   finished by a second kernel): issue the calls of one context on one stream at a time, or use a context per stream.
+ */
+int trs_locate_tracks(trs_ctx* ctx, const double* xyz_dev, const int32_t* track_dev, int n, int32_t* idx_dev,
+                      double* segment_dev, void* stream);
+
+/*
  * Replaces the speed-control tail of KerasPilot.step (keras_pilot.py:80-95,99-118,142-153) and
  * calcThrottle/calcBreak (utils/mapping.py:23-35) for N cars.
  *   cur_spd_dev (N) f64 `gym/speed`; model_spd_dev (N) f32 = the model's speed output (before x20);

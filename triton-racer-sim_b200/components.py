@@ -7,6 +7,7 @@ can be added to the reference's ``Car`` as they are.  All arithmetic runs in the
 
   ImgPreprocessing   components/img_preprocessing.py:9-108       cam/img -> cam/processed_img
   LocationTracker    components/track_data_process.py:68-107     gym/x, gym/y, gym/z -> loc/segment
+  MultiTrackLocationTracker  the same for cars on several tracks    gym/x, gym/y, gym/z, loc/track -> loc/segment
   SpeedControl       components/keras_pilot.py:80-95,99-118,142-153 + utils/mapping.py:23-35
   FrameNormalise     components/camera.py:36 + keras_pilot.py:49-50 / keras_train.py:41-42
   ControlMultiplexer components/controlmultiplexer.py:6-70        usr/*, ai/* -> mux/steering, mux/throttle, mux/breaking
@@ -239,6 +240,90 @@ class LocationTracker(Component):
 
     def getName(self):
         return 'Location Tracker'
+
+
+def _per_track(v, k: int, name: str):
+    vals = [v] * k if np.ndim(v) == 0 else list(v)
+    if len(vals) != k:
+        raise ValueError(f"{name}: one value per track ({k}), got {len(vals)}")
+    return (C.c_double * k)(*[float(x) for x in vals])
+
+
+class MultiTrackLocationTracker(Component):
+    """``LocationTracker`` for a batch of cars on several tracks: car i on ``track_data_paths[t_i]``.
+
+    Each car's segment is exactly what ``LocationTracker(track_data_paths[t_i], min_map[t_i], max_map[t_i])`` gives it, in one
+    stream-ordered call for the whole batch.  ``track_data_paths``: centre line files or (N, 3) point arrays (at most
+    ``nat.MAX_TRACKS``); ``min_map`` / ``max_map``: one value, or one per track.
+
+    Inputs ``gym/x, gym/y, gym/z, loc/track``; output ``loc/segment``.  ``loc/track`` is a key of this project, not of the reference
+    (where every car builds its own tracker, manage.py:97-99): the index of each car's track in ``track_data_paths``.
+    A track index outside ``[0, K)`` gives index -1 and segment NaN on the device path, and raises ``ValueError`` from the host forms.
+    """
+
+    def __init__(self, track_data_paths, min_map=0, max_map=10, device=None):
+        Component.__init__(self, inputs=['gym/x', 'gym/y', 'gym/z', 'loc/track'], outputs=['loc/segment'])
+        lines = []
+        for p in track_data_paths:
+            if isinstance(p, (str, bytes)) or hasattr(p, "__fspath__"):
+                with open(p, 'r') as input_file:
+                    p = json.load(input_file)
+            lines.append(np.ascontiguousarray(np.asarray(p, dtype=np.float64).reshape(-1, 3)))
+        k = len(lines)
+        if not 1 <= k <= nat.MAX_TRACKS:
+            raise ValueError(f"1 to {nat.MAX_TRACKS} tracks, got {k}")
+        self.min, self.max = min_map, max_map
+        self.n_tracks = k
+        self.device = _device_index(device)
+        self.ctx = nat.Context(self.device)
+        nat.check(self.ctx.lib.trs_set_tracks(self.ctx.handle, (C.c_void_p * k)(*[a.ctypes.data for a in lines]),
+                                              (C.c_int * k)(*[a.shape[0] for a in lines]), _per_track(min_map, k, "min_map"),
+                                              _per_track(max_map, k, "max_map"), k), "trs_set_tracks")
+        self.n_wp = [a.shape[0] for a in lines]
+
+    def locate_device(self, xyz: torch.Tensor, track: torch.Tensor, want_idx=True, want_segment=True):
+        """xyz (N,3) float64 and track (N,) int32 CUDA tensors -> (idx int32 (N,), segment float64 (N,)).  Enqueued on the current stream."""
+        if xyz.dtype != torch.float64 or xyz.dim() != 2 or xyz.shape[1] != 3:
+            raise ValueError(f"expected (N,3) float64, got {tuple(xyz.shape)} {xyz.dtype}")
+        xyz = xyz.contiguous()
+        _check_device_tensor(xyz, self.device, torch.float64, "xyz")
+        n = xyz.shape[0]
+        _check_device_tensor(track, self.device, torch.int32, "track")
+        if tuple(track.shape) != (n,):
+            raise ValueError(f"track must have shape ({n},), got {tuple(track.shape)}")
+        idx = torch.empty(n, dtype=torch.int32, device=xyz.device) if want_idx else None
+        seg = torch.empty(n, dtype=torch.float64, device=xyz.device) if want_segment else None
+        nat.check(self.ctx.lib.trs_locate_tracks(self.ctx.handle, _ptr(xyz), _ptr(track), n, _ptr(idx), _ptr(seg), _stream_ptr(self.device)),
+                  "trs_locate_tracks")
+        return idx, seg
+
+    def _host_tracks(self, track):
+        t = np.asarray(track)
+        if not np.issubdtype(t.dtype, np.integer):
+            raise ValueError(f"track indices must be integers, got {t.dtype}")
+        if t.size and (t.min() < 0 or t.max() >= self.n_tracks):
+            raise ValueError(f"track index outside [0, {self.n_tracks})")
+        return t.astype(np.int32)
+
+    def step(self, *args):
+        x, y, z, track = args[0], args[1], args[2], args[3]
+        if isinstance(x, torch.Tensor) and x.dim() >= 1:
+            xyz = torch.stack([x.to(torch.float64), y.to(torch.float64), z.to(torch.float64)], dim=1)
+            return self.locate_device(xyz, track, want_idx=False)[1],
+        dev = f"cuda:{self.device}"
+        if isinstance(x, np.ndarray) and x.ndim >= 1:
+            t = torch.from_numpy(np.ascontiguousarray(self._host_tracks(track))).to(dev)
+            xyz = torch.from_numpy(np.stack([x, y, z], axis=1).astype(np.float64)).to(dev)
+            return self.locate_device(xyz, t, want_idx=False)[1].cpu().numpy(),
+        t = torch.from_numpy(self._host_tracks([track])).to(dev)
+        xyz = torch.tensor([[float(x), float(y), float(z)]], dtype=torch.float64, device=dev)
+        return float(self.locate_device(xyz, t, want_idx=False)[1].item()),
+
+    def onShutdown(self):
+        self.ctx.close()
+
+    def getName(self):
+        return 'Multi-Track Location Tracker'
 
 
 class SpeedControl(Component):

@@ -206,4 +206,90 @@ inline std::vector<double> locg_distinct_quads(const double* wp, int n_wp)
     return quads;
 }
 
+// ---- several centre lines in one batch (trs_set_tracks / trs_locate_tracks, loc_tracks.cuh) ------------------------------------------------------
+// Every track keeps what trs_set_track builds for one: its distinct quads in order of first occurrence (the scan table) and, when locg_build gives
+// one, its cell-sorted quads and cell starts (the grid table).  The tracks' tables are concatenated; a descriptor per track holds the offsets.
+// Car i names its track t_i; the cars are bucketed by track (a stable counting sort) and each CTA of the walk takes a contiguous slice of the
+// bucketed cars, staging a track's grid table whenever its slice moves on to another track.
+struct LocTrack {
+    LocGrid g;                         // valid when grid_off >= 0
+    double min_map, max_map;
+    int n_wp;                          // points of the centre line (the divisor of the segment map)
+    int n_u;                           // distinct points
+    int scan_off;                      // first quad of its distinct points in the scan table
+    int grid_off;                      // first quad of its cell-sorted points in the grid table; -1: no grid (every car goes to the scan)
+    int cell_off;                      // first entry of its cell starts in the cell table
+    int pad_;
+};
+
+struct LocTracksHost {
+    std::vector<LocTrack> desc;
+    std::vector<double> scan, grid;    // quads
+    std::vector<int> cells;
+    size_t smem = 0;                   // the largest grid table in bytes (the walk's dynamic shared memory)
+};
+
+// Host: the tables of `k` centre lines (wp[t]: n_wp[t] x 3 f64).  A track whose grid would not fit `smem_limit` bytes, has non-finite
+// coordinates or fewer than LOCG_MIN_POINTS distinct points gets grid_off = -1.  Returns false when the concatenated tables would not be
+// addressable with int offsets.
+inline bool loct_build(const double* const* wp, const int* n_wp, const double* min_map, const double* max_map, int k, size_t smem_limit,
+                       LocTracksHost& out)
+{
+    out = LocTracksHost{};
+    out.desc.resize((size_t)k);
+    for (int t = 0; t < k; ++t) {
+        LocTrack& d = out.desc[(size_t)t];
+        d = LocTrack{};
+        const std::vector<double> quads = locg_distinct_quads(wp[t], n_wp[t]);
+        d.min_map = min_map[t]; d.max_map = max_map[t];
+        d.n_wp = n_wp[t]; d.n_u = (int)(quads.size() / 4);
+        if (out.scan.size() / 4 + quads.size() / 4 > (size_t)0x1fffffff) return false;
+        d.scan_off = (int)(out.scan.size() / 4);
+        out.scan.insert(out.scan.end(), quads.begin(), quads.end());
+        std::vector<double> sorted;
+        std::vector<int> start;
+        d.grid_off = -1;
+        if (locg_build(quads, smem_limit, d.g, sorted, start)) {
+            d.grid_off = (int)(out.grid.size() / 4);
+            d.cell_off = (int)out.cells.size();
+            out.grid.insert(out.grid.end(), sorted.begin(), sorted.end());
+            out.cells.insert(out.cells.end(), start.begin(), start.end());
+            out.smem = std::max(out.smem, locg_table_bytes(d.g));
+        } else {
+            d.g = LocGrid{};
+        }
+    }
+    return true;
+}
+
+// Bucket of a car's track index: t itself, or k for an index outside [0, k) (those cars get idx -1 / segment NaN and are not walked).
+LOCG_HD int loct_bucket(int32_t t, int k) { return (uint32_t)t < (uint32_t)k ? (int)t : k; }
+
+// Cars [b chunk, (b + 1) chunk) go to block b of the histogram and scatter passes: chunk a multiple of `step`, at most `max_blocks` blocks.
+LOCG_HD void loct_chunking(int n, int max_blocks, int step, int& chunk, int& nblk)
+{
+    const long long per = ((long long)n + max_blocks - 1) / max_blocks;
+    chunk = (int)((per + step - 1) / step * step);
+    if (chunk < step) chunk = step;
+    nblk = (int)(((long long)n + chunk - 1) / chunk);
+}
+
+// Positions [lo, hi) of the bucketed cars for CTA b of g, out of nv in-range cars.
+LOCG_HD void loct_slice(int nv, int b, int g, int& lo, int& hi)
+{
+    lo = (int)((long long)nv * b / g);
+    hi = (int)((long long)nv * (b + 1) / g);
+}
+
+// The track of bucketed position p < start[k]: the largest t < k with start[t] <= p (start: k + 1 bucket starts, ascending).
+LOCG_HD int loct_track_of(const int* start, int k, int p)
+{
+    int a = 0, b = k - 1;
+    while (a < b) {
+        const int m = (a + b + 1) >> 1;
+        if (start[m] <= p) a = m; else b = m - 1;
+    }
+    return a;
+}
+
 }  // namespace trs

@@ -24,6 +24,7 @@
 #include "jpeg_kernels.cuh"
 #include "jpeg_enc_kernels.cuh"
 #include "misc_kernels.cuh"
+#include "loc_tracks.cuh"
 #include "preproc_kernel.cuh"
 #include "preproc_fast.cuh"
 #include "preproc_bsw.cuh"
@@ -94,6 +95,16 @@ struct trs_ctx {
     int* defer_dev = nullptr;          // [0] = count, [1 ..] = cars k_locate_grid left to the warp-per-car kernel
     size_t defer_cap = 0;              // cars the list can hold
     double min_map = 0, max_map = 10;
+    // several tracks (trs_set_tracks / trs_locate_tracks, loc_tracks.cuh): concatenated tables, a descriptor per track, and the scratch of the
+    // large-batch path
+    int n_tracks = 0;
+    trs::LocTrack* tk_desc = nullptr;
+    double* tk_scan = nullptr;         // distinct quads of every track in order of first occurrence
+    double* tk_grid = nullptr;         // cell-sorted quads of the tracks that have a grid, nullptr: none has
+    int* tk_cells = nullptr;
+    size_t tk_smem = 0;                // the largest grid table (dynamic shared memory of k_locate_tracks_grid)
+    int* tk_scratch = nullptr;         // [0] list count | bucket starts (K + 2) | counts ((K + 1) x blocks) | bucketed cars (N) | list (N)
+    size_t tk_scratch_cap = 0;         // ints
     // host pipeline
     cudaStream_t hs[HOST_STREAMS] = {nullptr, nullptr, nullptr};
     uint8_t* st_in[HOST_STREAMS] = {nullptr, nullptr, nullptr};
@@ -508,6 +519,7 @@ int trs_ctx_destroy(trs_ctx* ctx)
     }
     if (ctx->host_entry) cudaEventDestroy(ctx->host_entry);
     cudaFree(ctx->wp_dev); cudaFree(ctx->wp_grid_dev); cudaFree(ctx->wp_cells_dev); cudaFree(ctx->defer_dev);
+    cudaFree(ctx->tk_desc); cudaFree(ctx->tk_scan); cudaFree(ctx->tk_grid); cudaFree(ctx->tk_cells); cudaFree(ctx->tk_scratch);
     cudaFree(ctx->stats_dev);
     cudaFree(ctx->jpg_blob); cudaFree(ctx->jpg_planes); cudaFree(ctx->jpg_meta);
     cudaFree(ctx->jpe_meta); cudaFree(ctx->jpe_sizes); cudaFree(ctx->jpe_offs); cudaFree(ctx->jpe_blob);
@@ -637,7 +649,8 @@ int trs_set_track(trs_ctx* ctx, const double* wp_xyz_host, int n_wp, double min_
         CU(cudaMemcpy(ctx->wp_grid_dev, sorted.data(), sizeof(double) * sorted.size(), cudaMemcpyHostToDevice));
         CU(cudaMalloc(&ctx->wp_cells_dev, sizeof(int) * start.size()));
         CU(cudaMemcpy(ctx->wp_cells_dev, start.data(), sizeof(int) * start.size(), cudaMemcpyHostToDevice));
-        CU(cudaFuncSetAttribute(trs::k_locate_grid, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)trs::locg_table_bytes(g)));
+        // the bound every table is built under, not this table's size: the attribute belongs to the kernel, and another context's table may be larger
+        CU(cudaFuncSetAttribute(trs::k_locate_grid, cudaFuncAttributeMaxDynamicSharedMemorySize, ctx->smem_optin - 1024));
         ctx->grid = g;
     }
     return 0;
@@ -694,6 +707,98 @@ int trs_locate(trs_ctx* ctx, const double* xyz_dev, int n, int32_t* idx_dev, dou
     trs::k_locate<<<grid, trs::LOC_THREADS, 0, (cudaStream_t)stream>>>(reinterpret_cast<const double4*>(ctx->wp_dev), ctx->n_wp_distinct, ctx->n_wp, ctx->min_map,
                                                                        ctx->max_map, xyz_dev, n, idx_dev, segment_dev);
     g_launches.fetch_add(1, std::memory_order_relaxed);
+    CU(cudaGetLastError());
+    return 0;
+}
+
+int trs_set_tracks(trs_ctx* ctx, const double* const* wp_xyz_host, const int* n_wp, const double* min_map, const double* max_map, int n_tracks)
+{
+    TRS_ENTER(ctx);
+    if (n_tracks < 1 || n_tracks > TRS_MAX_TRACKS) return fail(TRS_E_ARG, "%d tracks, outside [1,%d]", n_tracks, TRS_MAX_TRACKS);
+    if (!wp_xyz_host || !n_wp || !min_map || !max_map) return fail(TRS_E_ARG, "null pointer");
+    for (int t = 0; t < n_tracks; ++t)
+        if (!wp_xyz_host[t] || n_wp[t] <= 0) return fail(TRS_E_ARG, "track %d: empty centre line", t);
+    // per track what trs_set_track builds for one (loc_grid.h: first occurrences, and a grid where one fits), concatenated
+    trs::LocTracksHost h;
+    if (!trs::loct_build(wp_xyz_host, n_wp, min_map, max_map, n_tracks, (size_t)ctx->smem_optin - 1024, h))
+        return fail(TRS_E_ARG, "centre lines too large for one table");
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    ctx->n_tracks = 0;                                               // (no tracks if an upload below fails)
+    cudaFree(ctx->tk_desc); cudaFree(ctx->tk_scan); cudaFree(ctx->tk_grid); cudaFree(ctx->tk_cells);
+    ctx->tk_desc = nullptr; ctx->tk_scan = nullptr; ctx->tk_grid = nullptr; ctx->tk_cells = nullptr;
+    CU(cudaMalloc(&ctx->tk_desc, sizeof(trs::LocTrack) * h.desc.size()));
+    CU(cudaMemcpy(ctx->tk_desc, h.desc.data(), sizeof(trs::LocTrack) * h.desc.size(), cudaMemcpyHostToDevice));
+    CU(cudaMalloc(&ctx->tk_scan, sizeof(double) * h.scan.size()));
+    CU(cudaMemcpy(ctx->tk_scan, h.scan.data(), sizeof(double) * h.scan.size(), cudaMemcpyHostToDevice));
+    if (!h.grid.empty()) {
+        CU(cudaMalloc(&ctx->tk_grid, sizeof(double) * h.grid.size()));
+        CU(cudaMemcpy(ctx->tk_grid, h.grid.data(), sizeof(double) * h.grid.size(), cudaMemcpyHostToDevice));
+        CU(cudaMalloc(&ctx->tk_cells, sizeof(int) * h.cells.size()));
+        CU(cudaMemcpy(ctx->tk_cells, h.cells.data(), sizeof(int) * h.cells.size(), cudaMemcpyHostToDevice));
+        // the bound every table is built under, not this set's largest: the attribute belongs to the kernel, and other contexts may hold larger tables
+        CU(cudaFuncSetAttribute(trs::k_locate_tracks_grid, cudaFuncAttributeMaxDynamicSharedMemorySize, ctx->smem_optin - 1024));
+    }
+    ctx->tk_smem = h.smem;
+    ctx->n_tracks = n_tracks;
+    return 0;
+}
+
+int trs_locate_tracks(trs_ctx* ctx, const double* xyz_dev, const int32_t* track_dev, int n, int32_t* idx_dev, double* segment_dev, void* stream)
+{
+    TRS_ENTER(ctx);
+    if (!ctx->n_tracks) return fail(TRS_E_STATE, "trs_locate_tracks before trs_set_tracks");
+    if (n < 0) return fail(TRS_E_ARG, "negative n");
+    if (n == 0) return 0;
+    if (!xyz_dev || !track_dev || (!idx_dev && !segment_dev)) return fail(TRS_E_ARG, "null pointer");
+    const int k = ctx->n_tracks;
+    cudaStream_t st = (cudaStream_t)stream;
+    // small batches: a warp per car straight from the cars' order (the same crossover as trs_locate); large ones: bucket the cars by track, walk
+    // the grids, finish the cars the walk puts off with a warp per car.  TRS_LOCATE=warp|thread|grid forces one (thread: a scan per bucketed car).
+    const bool warp_per_car = ctx->sw.locate ? ctx->sw.locate == 1 : n < ctx->sm_count * 256;
+    if (warp_per_car) {
+        const int warps_per_block = trs::LOCW_THREADS / 32;
+        const int grid = std::min((n + warps_per_block - 1) / warps_per_block, ctx->sm_count * 8);
+        trs::k_locate_tracks_warp<<<grid, trs::LOCW_THREADS, 0, st>>>(ctx->tk_desc, k, ctx->tk_scan, xyz_dev, track_dev, n, idx_dev, segment_dev);
+        g_launches.fetch_add(1, std::memory_order_relaxed);
+        CU(cudaGetLastError());
+        return 0;
+    }
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    int chunk = 0, nblk = 0;
+    trs::loct_chunking(n, ctx->sm_count * 2, trs::LOCT_THREADS, chunk, nblk);
+    const size_t need = 1 + (size_t)(k + 2) + (size_t)(k + 1) * nblk + 2 * (size_t)n;
+    if (ctx->tk_scratch_cap < need) {
+        cudaFree(ctx->tk_scratch); ctx->tk_scratch = nullptr; ctx->tk_scratch_cap = 0;
+        CU(cudaMalloc(&ctx->tk_scratch, sizeof(int) * need));
+        ctx->tk_scratch_cap = need;
+    }
+    int* count = ctx->tk_scratch;
+    int* start = count + 1;
+    int* counts = start + (k + 2);
+    int* perm = counts + (size_t)(k + 1) * nblk;
+    int* list = perm + n;
+    trs::k_loct_hist<<<nblk, trs::LOCT_THREADS, sizeof(int) * (k + 1), st>>>(track_dev, n, k, chunk, nblk, counts, idx_dev, segment_dev);
+    trs::k_loct_scan<<<1, trs::LOCT_SCAN_THREADS, 0, st>>>(counts, nblk, k, n, start, count);
+    trs::k_loct_scatter<<<nblk, trs::LOCT_THREADS, sizeof(int) * (k + 1) * (1 + trs::LOCT_THREADS / 32), st>>>(track_dev, n, k, chunk, nblk, counts, perm);
+    g_launches.fetch_add(3, std::memory_order_relaxed);
+    CU(cudaGetLastError());
+    if (ctx->sw.locate == 2) {
+        const int grid = std::min((n + trs::LOCT_THREADS - 1) / trs::LOCT_THREADS, ctx->sm_count * 16);
+        trs::k_locate_tracks_scan<<<grid, trs::LOCT_THREADS, 0, st>>>(ctx->tk_desc, k, ctx->tk_scan, start, perm, xyz_dev, track_dev, idx_dev, segment_dev);
+        g_launches.fetch_add(1, std::memory_order_relaxed);
+        CU(cudaGetLastError());
+        return 0;
+    }
+    int per_sm = 0;
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, trs::k_locate_tracks_grid, trs::LOCG_THREADS, ctx->tk_smem));
+    per_sm = std::max(1, per_sm);
+    const int grid = std::min((n + trs::LOCG_THREADS - 1) / trs::LOCG_THREADS, ctx->sm_count * per_sm);
+    trs::k_locate_tracks_grid<<<grid, trs::LOCG_THREADS, ctx->tk_smem, st>>>(ctx->tk_desc, k, ctx->tk_grid, ctx->tk_cells, start, perm, xyz_dev,
+                                                                             idx_dev, segment_dev, list, count);
+    CU(cudaGetLastError());
+    trs::k_locate_tracks_warp<<<ctx->sm_count * 2, trs::LOCW_THREADS, 0, st>>>(ctx->tk_desc, k, ctx->tk_scan, xyz_dev, track_dev, n, idx_dev,
+                                                                               segment_dev, list, count);
+    g_launches.fetch_add(2, std::memory_order_relaxed);
     CU(cudaGetLastError());
     return 0;
 }
