@@ -113,6 +113,9 @@ int trs_set_preproc_params(trs_ctx* ctx, const trs_preproc_params* p);
  *   out_u8_dev  (N,H,W,3) u8  `cam/processed_img`            — nullable
  *   out_f32_dev (N,H,W,3) f32 `processed_img / 255`          — nullable
  *   stats_dev   TRS_STAT_COUNT x u64, accumulated atomically  — nullable
+ *   The kernels hand out frames to their CTAs from a per-context counter that is reset in stream order before each
+ *   launch: issue the calls of one context on one stream at a time, or use a context per stream.
+ *   (trs_preprocess_host keeps its own counters for its internal streams.)
  */
 int trs_preprocess(trs_ctx* ctx, const uint8_t* in_dev, int n, int h, int w,
                    uint8_t* out_u8_dev, float* out_f32_dev, unsigned long long* stats_dev,

@@ -74,6 +74,8 @@ class ImgPreprocessing(Component):
     The result is the one for *this* call.  The reference hands back the previous frame's result because its
     worker thread lags (img_preprocessing.py:18-35); ``emulate_latency=True`` reproduces that.
     ``normalised_key`` adds a second output: the float32 ``/255`` tensor the pilots consume (keras_pilot.py:49-50).
+    Calls of one component go to one CUDA stream at a time (its context hands out frames to the kernel's CTAs from one counter);
+    for concurrent streams use a component per stream.
     """
 
     def __init__(self, cfg={}, device=None, emulate_latency=False, normalised_key=None, collect_stats=False):

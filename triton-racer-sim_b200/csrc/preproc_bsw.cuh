@@ -23,6 +23,9 @@
 //    by frame parity, the candidate plane is handed back by a "hysteresis finished" barrier.
 //  * NSW store warps per CTA: two at 240x320 (two CTAs per SM), one at 120x160 (five compute warps, four CTAs per SM).
 //  * One named barrier per frame among the compute warps (before the hysteresis, whose row bands cut across the column blocks).
+//  * Frames come on demand (draw_frames, preproc_fast.cuh): the store warps draw frame j + 2 while the compute warps finish frame j and
+//    publish it in the frame ring before their "hysteresis finished" arrival of frame j, which the compute warps wait for in band 0 of
+//    frame j + 1, ahead of the last band, where the last warp out issues the copy of frame j + 2's first band.
 #pragma once
 #include "preproc_fast.cuh"
 
@@ -54,8 +57,8 @@ struct BswLayout {
     static constexpr int OFF_HUE = OFF_SDIV + 1024;
     static constexpr int OFF_BAR = OFF_HUE + 1024;                     // mbarriers: pixels, hysteresis finished, 2 per compute warp, 1 per mask slot
     static constexpr int NBAR = 2 + 2 * NCW + NSLOT;
-    static constexpr int OFF_SYNC = OFF_BAR + 8 * NBAR;                // strip-walk counter
-    static constexpr int OFF_RED = (OFF_SYNC + 16 + 15) & ~15;
+    static constexpr int OFF_SYNC = OFF_BAR + 8 * NBAR;                // strip-walk counter, then the frame ring (FRAME_RING u32)
+    static constexpr int OFF_RED = (OFF_SYNC + 16 + 4 * FRAME_RING + 15) & ~15;
     static constexpr int OFF_LUT = OFF_RED + 32 + 128;                 // brightness / contrast table (static, or rebuilt per frame)
     static constexpr int TOTAL = OFF_LUT + 256;
     static constexpr int THREADS = 32 * (NCW + NSW);
@@ -175,12 +178,15 @@ __global__ void __maxnreg__(MAXREG) k_preprocess_bsw(const __grid_constant__ Fas
     // mbarriers: [0] pixels of a band landed, [1] hysteresis of a frame finished, [2 + 2 w + q] strip walk of warp w for a band of parity q,
     // [2 + 2 NCW + s] the slab in mask slot s is written
     const uint32_t bar_pix = S.bar, bar_p3 = S.bar + 8, bar_p1 = S.bar + 16, bar_slot = bar_p1 + 16 * NCW;
-    const uint32_t a_cnt = sb + L::OFF_SYNC;
+    const uint32_t a_cnt = sb + L::OFF_SYNC, a_ring = a_cnt + 16;
     const uint32_t a_stash = sb + L::OFF_STASH, a_zero = a_stash + NCW * 8 * L::STASH_LANE;
     Dims Dm;
     Dm.h = H; Dm.w = W; Dm.mag_stride = W + 4; Dm.plane_bytes = L::MASKP;      // (the walks use plane_bytes for the stride between colour ranges only)
-    const int nfr = (int)blockIdx.x < p.n ? (p.n - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x : 0;
+    const uint32_t n = (uint32_t)p.n;
+    static_assert(NB >= 2, "the last band reads the next frame after band 0's wait for the hysteresis of the frame before");
 
+    uint32_t ticket = 0;
+    if (tid == NC) ticket = draw_frames(p);                        // frame 1, in flight during the set-up
     init_tables<NR, F0, F1>(p, S, tid, NT);
     stats_zero(S, tid);
     for (int i = tid; i < 2 * R + 2; i += NT) {                   // the zero left of pixel 0 (element 3) and right of pixel W - 1 (element 0 of the next row)
@@ -193,6 +199,7 @@ __global__ void __maxnreg__(MAXREG) k_preprocess_bsw(const __grid_constant__ Fas
     for (int i = tid; i < L::STASH_ROW / 4; i += NT) sts32(a_zero + 4 * i, 0);
     if (tid < L::NBAR) mbar_init(S.bar + 8 * tid, tid >= 2 + 2 * NCW ? (uint32_t)NSW : 1u);      // a slot's barrier takes every store warp
     asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    if (tid == NC) { sts32(a_ring, blockIdx.x); sts32(a_ring + 4, ticket); }
     __syncthreads();
 
     // pixel rows of band b: [max(R b - 1, 0), min(R b + R + 1, H))
@@ -210,17 +217,21 @@ __global__ void __maxnreg__(MAXREG) k_preprocess_bsw(const __grid_constant__ Fas
         M.store_lane = !(lane & 1);
         const uint32_t my_slot = a_stash + (uint32_t)(warp * 8 + (lane & 7)) * L::STASH_LANE;
         const uint32_t my_bar = bar_p1 + 16 * warp;
-        if (tid == 0 && nfr > 0) issue_band(blockIdx.x, 0);
+        if (tid == 0 && blockIdx.x < n) issue_band(blockIdx.x, 0);
         uint32_t gb = 0;                                          // bands finished by this warp since the kernel started
         int slot = 0;                                             // gb % NSLOT: the mask slot of the band
         uint32_t round = 0;                                       // gb / NSLOT: how often the slot has been used before
+        // the CTA's frame k (k >= 2) is published before the store warps' arrival on bar_p3 for frame k - 2, which every compute thread
+        // waits for in band 0 of frame k - 1; it is read in the last band of frame k - 1 (the last warp out) and at the top of iteration k.
+        // Frames 0 and 1: set-up barrier.
 #pragma unroll 1
-        for (int j = 0; j < nfr; ++j) {
-            const size_t f = blockIdx.x + (size_t)j * gridDim.x;
+        for (int j = 0;; ++j) {
+            const uint32_t f = ring_frame(a_ring, j);
+            if (f >= n) break;
             const uint32_t a_edge = (j & 1) ? S.edge2 : S.edge;
             if (LUT && p.dynamic) {
                 constexpr int Y0 = H < 40 ? H : 40, Y1 = H < 119 ? H : 119, NTRI = (Y1 - Y0) * L::ROWB / 12;      // groups of four pixels = three words
-                const uint32_t* roi = reinterpret_cast<const uint32_t*>(p.in + f * frame_bytes + (size_t)Y0 * L::ROWB);
+                const uint32_t* roi = reinterpret_cast<const uint32_t*>(p.in + (size_t)f * frame_bytes + (size_t)Y0 * L::ROWB);
                 uint32_t c0 = 0, c1 = 0, c2 = 0;
 #pragma unroll 4
                 for (int i = tid; i < NTRI; i += NC) {
@@ -266,7 +277,7 @@ __global__ void __maxnreg__(MAXREG) k_preprocess_bsw(const __grid_constant__ Fas
                     mbar_arrive(my_bar + 8 * (gb & 1u));
                     if (atom_inc_acq_rel(a_cnt) == (uint32_t)NCW * (gb + 1) - 1) {      // the last warp out: the band's pixels are dead
                         if (b + 1 < NB) issue_band(f, b + 1);
-                        else if (j + 1 < nfr) issue_band(f + gridDim.x, 0);
+                        else if (const uint32_t fn = ring_frame(a_ring, j + 1); fn < n) issue_band(fn, 0);
                     }
                 }
                 // the neighbours' magnitudes of this band (barrier gb & 1 of a warp is in its phase gb >> 1)
@@ -293,9 +304,12 @@ __global__ void __maxnreg__(MAXREG) k_preprocess_bsw(const __grid_constant__ Fas
         Dims Ds = Dm;
         Ds.h = R;
         int slot = 0;
+        // slot j was written by thread NC two frames ago, before a barrier of both store warps
 #pragma unroll 1
-        for (int j = 0; j < nfr; ++j) {
-            const size_t f = blockIdx.x + (size_t)j * gridDim.x;
+        for (int j = 0;; ++j) {
+            const uint32_t f = ring_frame(a_ring, j);
+            if (f >= n) break;
+            if (st == 0) ticket = draw_frames(p);                 // frame j + 2: published after this frame's hysteresis
             const uint32_t a_edge = (j & 1) ? S.edge2 : S.edge;
             bar_sync(2, NT);
             int sw = 0;                                           // growth across the compute warps' row bands (usually one checking pass)
@@ -306,9 +320,12 @@ __global__ void __maxnreg__(MAXREG) k_preprocess_bsw(const __grid_constant__ Fas
                 count_planes<0, true>(p, S, S.cand, a_edge, 0u, 0, H * ww, st, NS);
                 bar_sync(4, NS);
             }
-            if (st == 0) mbar_arrive(bar_p3);                     // (the barriers above order both store warps' reads of the candidate plane)
-            uint8_t* gu8 = p.out_u8 ? p.out_u8 + f * frame_bytes : nullptr;
-            float* gf32 = p.out_f32 ? p.out_f32 + f * frame_bytes : nullptr;
+            if (st == 0) {                                        // (the barriers above order both store warps' reads of the candidate plane)
+                sts32(a_ring + 4 * (uint32_t)((j + 2) % FRAME_RING), ticket);      // (slot of frame j - 2: every reader is past it)
+                mbar_arrive(bar_p3);
+            }
+            uint8_t* gu8 = p.out_u8 ? p.out_u8 + (size_t)f * frame_bytes : nullptr;
+            float* gf32 = p.out_f32 ? p.out_f32 + (size_t)f * frame_bytes : nullptr;
 #pragma unroll 1
             for (int b = 0; b < NB; ++b) {
                 // the slab's sources: rows R b .. of the frame's edge plane, the band's slot of the mask ring

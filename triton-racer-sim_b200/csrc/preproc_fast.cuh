@@ -1403,11 +1403,24 @@ __global__ void __launch_bounds__(FAST_MAX_THREADS, 2) k_preprocess_banded(const
 //            may finish frame j + 1 before the compute warps have asked about frame j - with a brightness / contrast table the compute warps
 //            first wait for the tail copy the store warps issue and then rewrite the frame - and a second round of arrivals on a named
 //            barrier whose first round is still open completes it early and strands the late compute warps.)
+//            Frames come on demand (draw_frames): the store warps draw frame j + 3 while they work on frame j and publish it in the frame
+//            ring before that same bar_free arrival, which is where the compute warps learn it (they need frame j + 1 after P1 of frame j).
 // Compute-only phases use named barrier 1.
 // =========================================================================================================
 enum { SW_COMPUTE_THREADS = 320, SW_THREADS = 384, SW_MAXREG = 80 };      // register allocation rounds a CTA up to a multiple of 4 warps
 
 __device__ __forceinline__ void bar_arrive(int id, int nthreads) { asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(nthreads) : "memory"); }
+
+// Frames on demand (k_preprocess_sw, k_preprocess_bsw).  What a frame costs depends on its content, so a fixed stride (CTA b takes b, b + G,
+// b + 2G, ...) leaves the launch waiting for the CTAs that drew the slow frames: a batch of interleaved sources with a period that divides G
+// puts every CTA on one kind of frame.  Instead a CTA's first frame is blockIdx.x and each further one is gridDim.x + a ticket from the
+// launch's counter.  One thread per CTA draws the tickets, one after the other, so a CTA's frames increase and the first one >= n ends its
+// loop: every frame is processed exactly once whatever the timing, and outputs are addressed by frame, so results do not depend on the order.
+// The tickets are drawn ahead and published in a ring of FRAME_RING frame indices in shared memory (slot j % FRAME_RING: the CTA's frame j),
+// handed over by barriers the roles already share (DESIGN.md §4.9): no warp waits for the atomic's round trip.
+enum { FRAME_RING = 4 };
+__device__ __forceinline__ uint32_t draw_frames(const PreKParams& p, uint32_t k = 1) { return gridDim.x + atomicAdd(p.frame_ctr, k); }
+__device__ __forceinline__ uint32_t ring_frame(uint32_t a_ring, int j) { return lds32(a_ring + 4 * (uint32_t)(j % FRAME_RING)); }
 
 // H, W > 0: the frame size is a compile-time constant (the host launches such a variant only for exactly that size, with the geometry
 // sw_static_geometry_ok() accepts); H = W = 0: any size that fits.
@@ -1441,11 +1454,14 @@ __global__ void __maxnreg__(SW_MAXREG) k_preprocess_sw(const __grid_constant__ F
     const uint32_t frame_bytes = (uint32_t)h * w * 3;
     const int plane_words = h * ww;
     const int NC = SW_COMPUTE_THREADS;
-    const int nfr = (int)blockIdx.x < p.n ? (p.n - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x : 0;
+    const uint32_t n = (uint32_t)p.n;
     const uint32_t mask_set_bytes = (uint32_t)(NR * Dm.plane_bytes);
     const uint32_t main_bytes = frame_bytes - (uint32_t)tail_bytes;
     const uint32_t bar_main = S.bar, bar_tail = S.bar + 8, bar_free = S.bar + 16;      // bar_free + 8 q: plane set q has been written out
+    const uint32_t a_ring = S.bar + 32;                                                  // frame ring (the barrier block's free half)
 
+    uint32_t ticket = 0;
+    if (tid == NC) ticket = draw_frames(p, 2);                    // frames 1 and 2, in flight during the set-up
     init_tables<NR, F0, F1>(p, S, tid, nthr);
     stats_zero(S, tid);
     zero_mag_borders(S.mag[0], h, w, Dm.mag_stride, tid, nthr);
@@ -1455,6 +1471,7 @@ __global__ void __maxnreg__(SW_MAXREG) k_preprocess_sw(const __grid_constant__ F
         mbar_init(bar_free, (SW_THREADS - SW_COMPUTE_THREADS) / 32); mbar_init(bar_free + 8, (SW_THREADS - SW_COMPUTE_THREADS) / 32);      // one arrival per store warp
         asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
     }
+    if (tid == NC) { sts32(a_ring, blockIdx.x); sts32(a_ring + 4, ticket); sts32(a_ring + 8, ticket + 1); }
     __syncthreads();
 
     if (warp < (NC >> 5)) {
@@ -1466,7 +1483,7 @@ __global__ void __maxnreg__(SW_MAXREG) k_preprocess_sw(const __grid_constant__ F
         const int tail_row = (int)(main_bytes / (uint32_t)(w * 3));
         int tail_k = tail_row - (nsegs - 1) * seg_rows + 1;
         tail_k = tail_k < 0 ? 0 : (tail_k / 3) * 3;
-        if (tid == 0 && nfr > 0) {
+        if (tid == 0 && blockIdx.x < n) {
             const uint8_t* src = p.in + (size_t)blockIdx.x * frame_bytes;
             issue_frame_piece(S.pix[0], src, 0, main_bytes, bar_main);
             if (tail_bytes) issue_frame_piece(S.pix[0], src, main_bytes, frame_bytes, bar_tail);
@@ -1479,8 +1496,9 @@ __global__ void __maxnreg__(SW_MAXREG) k_preprocess_sw(const __grid_constant__ F
 #else
 #define TRS_TICK(v)
 #endif
-        for (int j = 0; j < nfr; ++j) {
-            const size_t f = blockIdx.x + (size_t)j * gridDim.x;
+        // the CTA's frame k (k >= 3) is published before the store warps' arrival on bar_free for frame k - 3, which every compute thread
+        // waits for before P1 of frame k - 1; it is read after that P1 (thread 0) and at the top of iteration k.  Frames 0..2: set-up barrier.
+        for (int j = 0; ring_frame(a_ring, j) < n; ++j) {
             const uint32_t a_mask = S.mask + (j & 1) * mask_set_bytes;
             const uint32_t a_edge = (j & 1) ? S.edge2 : S.edge;
             TRS_TICK(tk0);
@@ -1496,8 +1514,10 @@ __global__ void __maxnreg__(SW_MAXREG) k_preprocess_sw(const __grid_constant__ F
             phase ^= 1u;
             bar_sync(1, NC);
             TRS_TICK(tk4);
-            if (tid == 0 && j + 1 < nfr)                                 // pixels are dead: prefetch the next frame (all but its tail)
-                issue_frame_piece(S.pix[0], p.in + (f + gridDim.x) * frame_bytes, 0, main_bytes, bar_main);
+            if (tid == 0) {                                              // pixels are dead: prefetch the next frame (all but its tail)
+                const uint32_t fn = ring_frame(a_ring, j + 1);
+                if (fn < n) issue_frame_piece(S.pix[0], p.in + (size_t)fn * frame_bytes, 0, main_bytes, bar_main);
+            }
             p2_nms<(STATIC ? sw_seg_rows<(STATIC ? H : 32), (STATIC ? W : 32)>() : 0), false>(P, Dm, S.mag[0], S.cand, a_edge, S, M, seg_rows);
             bar_sync(1, NC);
             TRS_TICK(tk5);
@@ -1520,8 +1540,11 @@ __global__ void __maxnreg__(SW_MAXREG) k_preprocess_sw(const __grid_constant__ F
 #undef TRS_TICK
     } else {
         // ------------------------------------------------ store warps -------------------------------------------------
-        for (int j = 0; j < nfr; ++j) {
-            const size_t f = blockIdx.x + (size_t)j * gridDim.x;
+        // slots j and j + 1 were written by thread NC at least two frames ago, before a barrier of both store warps
+        for (int j = 0;; ++j) {
+            const uint32_t f = ring_frame(a_ring, j);
+            if (f >= n) break;
+            if (tid == NC) ticket = draw_frames(p);                      // frame j + 3: published after this frame's output
             uint32_t pa[3];
             plane_sources(p, (j & 1) ? S.edge2 : S.edge, S.mask + (j & 1) * mask_set_bytes, Dm.plane_bytes, pa);
             bar_sync(2, SW_THREADS);
@@ -1538,12 +1561,15 @@ __global__ void __maxnreg__(SW_MAXREG) k_preprocess_sw(const __grid_constant__ F
                     count_planes<NR, true>(p, S, S.cand, a_edge, a_mask, Dm.plane_bytes, plane_words, tid - NC, NS);
                     bar_sync(4, NS);
                 }
-                if (tid == NC && tail_bytes && j + 1 < nfr)              // the candidate plane is dead: fetch the tail it was sitting in
-                    issue_frame_piece(S.pix[0], p.in + (f + gridDim.x) * frame_bytes, main_bytes, frame_bytes, bar_tail);
+                if (tid == NC && tail_bytes) {                           // the candidate plane is dead: fetch the tail it was sitting in
+                    const uint32_t fn = ring_frame(a_ring, j + 1);
+                    if (fn < n) issue_frame_piece(S.pix[0], p.in + (size_t)fn * frame_bytes, main_bytes, frame_bytes, bar_tail);
+                }
             }
-            p4_output(P, Dm, pa, S.pix[0], p.out_u8 ? p.out_u8 + f * frame_bytes : nullptr, p.out_f32 ? p.out_f32 + f * frame_bytes : nullptr, tid - NC,
-                      SW_THREADS - NC);
+            p4_output(P, Dm, pa, S.pix[0], p.out_u8 ? p.out_u8 + (size_t)f * frame_bytes : nullptr, p.out_f32 ? p.out_f32 + (size_t)f * frame_bytes : nullptr,
+                      tid - NC, SW_THREADS - NC);
             __syncwarp();
+            if (tid == NC) sts32(a_ring + 4 * (uint32_t)((j + 3) % FRAME_RING), ticket);      // (slot of frame j - 1: every reader is past it)
             if (lane == 0) mbar_arrive(bar_free + 8 * (j & 1));          // (use k of a plane set's barrier is its phase k: frame j + 2 waits for phase j >> 1)
         }
         if (p.stats) {                                                   // the store warps are the last to touch the counters

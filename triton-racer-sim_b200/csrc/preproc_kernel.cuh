@@ -32,6 +32,7 @@ struct PreKParams {
     unsigned long long* stats;
     uint16_t* dbg_mag;      // debug taps: frame 0 only
     uint8_t* dbg_map;
+    uint32_t* frame_ctr;    // frame tickets of this launch (store-warp kernels, preproc_fast.cuh draw_frames): zeroed in stream order before it
     int n, h, w;
     int band_h;             // image rows per band
     int row_stride;         // bytes per smem pixel row (16-byte multiple; pixels start at +16)

@@ -86,6 +86,7 @@ struct trs_ctx {
     bool have_params = false;
     trs_preproc_params user{};
     trs::PreKParams kp{};              // derived, geometry fields filled per call
+    uint32_t* frame_ctr = nullptr;     // frame tickets of the store-warp kernels, one per launch slot: [0] trs_preprocess, [1 + s] staging set s
     // track
     double* wp_dev = nullptr;          // distinct waypoints in order of first occurrence: (x, y, z, original index) quads
     int n_wp = 0, n_wp_distinct = 0;
@@ -249,14 +250,16 @@ int launch_fast_tf(const trs::FastParams& fp, int grid, cudaStream_t st)
 {
     if (EDGE && fp.use_store_warp) {
         // the reference's camera size with its default colour ranges (core/config.py:8-9,23) gets the variant with compile-time dimensions
+        cudaError_t e = cudaMemsetAsync(fp.k.frame_ctr, 0, sizeof(uint32_t), st);      // the launch's frame tickets start at 0
+        if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(frame counter)");
         if (NR == 2 && F0 >= 0 && trs::sw_static_geometry_ok<120, 160>(fp.g, fp.k.h, fp.k.w)) {
             auto kern = trs::k_preprocess_sw<NR, F0, F1, (NR == 2 && F0 >= 0 ? 120 : 0), (NR == 2 && F0 >= 0 ? 160 : 0)>;
-            cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, fp.g.total);
+            e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, fp.g.total);
             if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(sw 120x160)");
             kern<<<grid, trs::SW_THREADS, fp.g.total, st>>>(fp);
             return 0;
         }
-        cudaError_t e = cudaFuncSetAttribute(trs::k_preprocess_sw<NR, F0, F1>, cudaFuncAttributeMaxDynamicSharedMemorySize, fp.g.total);
+        e = cudaFuncSetAttribute(trs::k_preprocess_sw<NR, F0, F1>, cudaFuncAttributeMaxDynamicSharedMemorySize, fp.g.total);
         if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(sw)");
         trs::k_preprocess_sw<NR, F0, F1><<<grid, trs::SW_THREADS, fp.g.total, st>>>(fp);
         return 0;
@@ -303,6 +306,8 @@ int launch_bsw(trs_ctx* ctx, const trs::FastParams& fp, int n, cudaStream_t st)
     if (per_sm < 1) return 0;
     int grid = ctx->sm_count * per_sm;
     if (grid > n) grid = n;
+    e = cudaMemsetAsync(fp.k.frame_ctr, 0, sizeof(uint32_t), st);                  // the launch's frame tickets start at 0
+    if (e != cudaSuccess) { cuda_fail(e, "cudaMemsetAsync(frame counter)"); return -100 - (int)e; }
     kern<<<grid, L::THREADS, L::TOTAL, st>>>(fp);
     g_launches.fetch_add(1, std::memory_order_relaxed);
     e = cudaGetLastError();
@@ -412,14 +417,16 @@ int try_launch_fast(trs_ctx* ctx, const trs::PreKParams& k, int n, int h, int w,
     return 1;
 }
 
+// ctr_slot: the context's frame counter this launch may use (trs_ctx::frame_ctr): launches that can overlap on the device take different slots
 int launch_preprocess(trs_ctx* ctx, const uint8_t* in, int n, int h, int w, uint8_t* out_u8, float* out_f32,
-                      unsigned long long* stats, uint16_t* dbg_mag, uint8_t* dbg_map, bool force_edge, cudaStream_t st)
+                      unsigned long long* stats, uint16_t* dbg_mag, uint8_t* dbg_map, bool force_edge, cudaStream_t st, int ctr_slot)
 {
     trs::PreKParams k = ctx->kp;
     if (force_edge && !k.edge_enabled) { k.edge_enabled = 1; }
     if (!dbg_mag && !dbg_map) {
         trs::PreKParams kf = k;
         kf.in = in; kf.out_u8 = out_u8; kf.out_f32 = out_f32; kf.stats = stats; kf.dbg_mag = nullptr; kf.dbg_map = nullptr;
+        kf.frame_ctr = ctx->frame_ctr + ctr_slot;
         kf.n = n; kf.h = h; kf.w = w;
         kf.word_io = ((w * 3) % 4 == 0) && (((uintptr_t)in & 15) == 0) && (!out_u8 || ((uintptr_t)out_u8 & 15) == 0) &&
                      (!out_f32 || ((uintptr_t)out_f32 & 15) == 0) && (((size_t)h * w * 3) % 4 == 0);
@@ -502,6 +509,11 @@ int trs_ctx_create(int device, trs_ctx** out)
     c->sw.resize_gather = getenv("TRS_RESIZE_GATHER") != nullptr;
     if (const char* e = getenv("TRS_LOCATE")) c->sw.locate = e[0] == 'w' ? 1 : (e[0] == 'g' ? 3 : 2);
     if (const char* e = getenv("TRS_HOST_CHUNK_MB")) { const int mb = atoi(e); if (mb > 0) c->sw.host_chunk_bytes = (size_t)mb << 20; }
+    {
+        TrsDeviceGuard guard(device);
+        e = guard.err != cudaSuccess ? guard.err : cudaMalloc(&c->frame_ctr, sizeof(uint32_t) * (1 + HOST_STREAMS));
+        if (e != cudaSuccess) { delete c; return cuda_fail(e, "cudaMalloc(frame counters)"); }
+    }
     trs_preproc_params d;
     default_params(&d);
     derive_params(c, &d);
@@ -518,6 +530,7 @@ int trs_ctx_destroy(trs_ctx* ctx)
         cudaFree(ctx->st_in[i]); cudaFree(ctx->st_u8[i]); cudaFree(ctx->st_f32[i]);
     }
     if (ctx->host_entry) cudaEventDestroy(ctx->host_entry);
+    cudaFree(ctx->frame_ctr);
     cudaFree(ctx->wp_dev); cudaFree(ctx->wp_grid_dev); cudaFree(ctx->wp_cells_dev); cudaFree(ctx->defer_dev);
     cudaFree(ctx->tk_desc); cudaFree(ctx->tk_scan); cudaFree(ctx->tk_grid); cudaFree(ctx->tk_cells); cudaFree(ctx->tk_scratch);
     cudaFree(ctx->stats_dev);
@@ -552,14 +565,14 @@ int trs_preprocess(trs_ctx* ctx, const uint8_t* in_dev, int n, int h, int w, uin
     if (n == 0 || h == 0 || w == 0) return 0;
     if (!in_dev) return fail(TRS_E_ARG, "null input");
     if (!out_u8_dev && !out_f32_dev && !stats_dev) return fail(TRS_E_ARG, "no output requested");
-    return launch_preprocess(ctx, in_dev, n, h, w, out_u8_dev, out_f32_dev, stats_dev, nullptr, nullptr, false, (cudaStream_t)stream);
+    return launch_preprocess(ctx, in_dev, n, h, w, out_u8_dev, out_f32_dev, stats_dev, nullptr, nullptr, false, (cudaStream_t)stream, 0);
 }
 
 int trs_debug_canny_stages(trs_ctx* ctx, const uint8_t* in_dev, int h, int w, uint16_t* mag_dev, uint8_t* map_dev, void* stream)
 {
     TRS_ENTER(ctx);
     if (!in_dev || h <= 0 || w <= 0) return fail(TRS_E_ARG, "bad argument");
-    return launch_preprocess(ctx, in_dev, 1, h, w, nullptr, nullptr, nullptr, mag_dev, map_dev, true, (cudaStream_t)stream);
+    return launch_preprocess(ctx, in_dev, 1, h, w, nullptr, nullptr, nullptr, mag_dev, map_dev, true, (cudaStream_t)stream, 0);
 }
 
 int trs_normalise(trs_ctx* ctx, const uint8_t* in_dev, int n, int h_in, int w_in, int roi_y0, int roi_y1, int roi_x0, int roi_x1,
@@ -1245,7 +1258,7 @@ int trs_preprocess_host(trs_ctx* ctx, const uint8_t* in_host, int n, int h, int 
         CUD(cudaMemcpyAsync(ctx->st_in[s], in_host + f0 * fb, cn * fb, cudaMemcpyHostToDevice, st));
         uint8_t* du8 = out_u8_host ? ctx->st_u8[s] : nullptr;
         float* df32 = keep_f32_dev ? keep_f32_dev + f0 * fb : (need_f32 ? ctx->st_f32[s] : nullptr);
-        rc = launch_preprocess(ctx, ctx->st_in[s], (int)cn, h, w, du8, df32, stats_host ? ctx->stats_dev : nullptr, nullptr, nullptr, false, st);
+        rc = launch_preprocess(ctx, ctx->st_in[s], (int)cn, h, w, du8, df32, stats_host ? ctx->stats_dev : nullptr, nullptr, nullptr, false, st, 1 + s);
         if (rc) return drain(rc);
         if (out_u8_host) CUD(cudaMemcpyAsync(out_u8_host + f0 * fb, du8, cn * fb, cudaMemcpyDeviceToHost, st));
         if (need_f32) CUD(cudaMemcpyAsync(out_f32_host + f0 * fb, df32, cn * fb * 4, cudaMemcpyDeviceToHost, st));
