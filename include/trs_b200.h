@@ -221,7 +221,14 @@ int trs_pwm_map(trs_ctx* ctx, const double* val_dev, int n, double min_map, doub
  *   out_u8_dev    (N, h, w, 3) uint8 RGB on the device; every file must be h x w
  * Parses on the host, uploads the files (about 5 KB per 120x160 record instead of 57.6 KB of pixels), decodes on the GPU;
  * synchronises `stream` before returning (the staging buffers are reused by the next call).
- * TRS_E_RANGE: a file is not a baseline 4:2:0 JPEG of the stated size (the message names the record).
+ * Also accepted: 4:2:2 and 4:4:4 (one subsampling per batch), optimised Huffman tables, OpenCV's files, APPn / COM segments,
+ * 0xFF fill bytes, DRI with interval 0, bytes after EOI.  Refused: progressive, greyscale, 4:1:1 / 4:4:0, restart intervals,
+ * separate Cb / Cr quantisation tables.
+ * A batch holds at most 64 distinct table sets (quantisation + Huffman tables).  Files written with optimised Huffman tables
+ * (Pillow optimize=True, OpenCV IMWRITE_JPEG_OPTIMIZE) carry tables of their own, so each such file counts one set: a batch of
+ * more than 64 of them is refused.
+ * TRS_E_RANGE: a file is not a supported JPEG of the stated size (the message names the lowest such record), or the batch has
+ * more than 64 distinct table sets.
  */
 int trs_jpeg_decode_host(trs_ctx* ctx, const uint8_t* blob_host, const unsigned long long* offsets_host, int n, int h, int w,
                          uint8_t* out_u8_dev, void* stream);
@@ -231,7 +238,8 @@ int trs_jpeg_decode_host(trs_ctx* ctx, const uint8_t* blob_host, const unsigned 
  *   Image.open(BytesIO(base64.b64decode(json_packet["image"])))     TritonRacerSim/components/gyminterface.py:96-99
  * text_host holds the N base64 strings back to back (standard alphabet, '=' padding optional, white space ignored),
  * offsets_host N + 1 byte offsets into it.  The strings are decoded on the host (threads) and the JPEG files go through the same
- * path as trs_jpeg_decode_host.  TRS_E_RANGE: a string is not valid base64 or not a supported JPEG of the stated size.
+ * path as trs_jpeg_decode_host (and its 64-set limit).  TRS_E_RANGE: a string is not valid base64 (the message names the lowest
+ * such packet) or not a supported JPEG of the stated size.
  */
 int trs_telemetry_decode_host(trs_ctx* ctx, const char* text_host, const unsigned long long* offsets_host, int n, int h, int w,
                               uint8_t* out_u8_dev, void* stream);
