@@ -122,6 +122,31 @@ int trs_preprocess(trs_ctx* ctx, const uint8_t* in_dev, int n, int h, int w,
                    void* stream);
 
 /*
+ * Several preprocessing configurations in one batch: what one ImgPreprocessing per car does when the cars come from simulators
+ * on different tracks, each with its own myconfig.json (manage.py:91-94).  Upload n_cfgs configurations,
+ * 1 <= n_cfgs <= TRS_MAX_PREPROC_CONFIGS, each validated and derived as trs_set_preproc_params does it (an invalid entry fails
+ * the whole call and leaves the previous set).  Replaces the previous set; the context's single configuration
+ * (trs_set_preproc_params, used by trs_preprocess and trs_preprocess_host) is left as it is.
+ */
+#define TRS_MAX_PREPROC_CONFIGS 16
+int trs_set_preproc_configs(trs_ctx* ctx, const trs_preproc_params* cfgs, int n_cfgs);
+
+/*
+ * trs_preprocess for N frames, frame i with configuration cfg_dev[i]: its outputs are bit for bit what trs_preprocess
+ * writes for that frame with that configuration alone.
+ *   in_dev (N,H,W,3) u8; cfg_dev (N) i32; out_u8_dev (N,H,W,3) u8 — nullable; out_f32_dev (N,H,W,3) f32 — nullable.
+ *   stats_dev   n_cfgs x TRS_STAT_COUNT u64 — nullable: row c holds configuration c's counters over its own frames
+ *               (the range slots keep their meaning per configuration), accumulated atomically.
+ *   A frame whose index is outside [0, n_cfgs) gets u8 0 and f32 NaN (nothing is reported to the host: the call does not
+ *   synchronise).  One kernel launch per configuration (plus the bucketing of the frames by configuration), enqueued on
+ *   `stream`; no allocation after the first call of a given N, so the call can be captured in a CUDA graph.  The bucketed
+ *   frames and the frame counters are per-context scratch: issue the calls of one context on one stream at a time, or use
+ *   a context per stream.
+ */
+int trs_preprocess_configs(trs_ctx* ctx, const uint8_t* in_dev, const int32_t* cfg_dev, int n, int h, int w,
+                           uint8_t* out_u8_dev, float* out_f32_dev, unsigned long long* stats_dev, void* stream);
+
+/*
  * Replaces the camera resize (camera.py:36, nearest neighbour), a rows/cols window crop and the
  * float normalisation (keras_pilot.py:49-50, keras_train.py:41-42) for N frames.
  *   in_dev (N,h_in,w_in,3) u8; window rows [roi_y0,roi_y1) cols [roi_x0,roi_x1) of the source;

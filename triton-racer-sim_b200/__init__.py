@@ -2,8 +2,8 @@
 
 Import as ``triton_racer_sim_b200`` (shim at the repo root).  Public names mirror the reference:
 ``Component`` (components/component.py), ``ImgPreprocessing`` (components/img_preprocessing.py),
-``LocationTracker`` (components/track_data_process.py:68-107) and ``MultiTrackLocationTracker`` (the same for a batch of cars
-on several tracks), plus the batched pilot glue
+``LocationTracker`` (components/track_data_process.py:68-107) and ``MultiTrackLocationTracker`` / ``MultiTrackImgPreprocessing``
+(the same for a batch of cars on several tracks, each track with its own centre line / preprocessing configuration), plus the batched pilot glue
 ``SpeedControl`` / ``FrameNormalise`` (components/keras_pilot.py:49-50,80-95,142-153; camera.py:36) and the per-car control
 post-processing ``ControlMultiplexer`` / ``DriverAssistance`` / ``three_segment_map`` (components/controlmultiplexer.py,
 components/driver_assistance.py, utils/mapping.py:9-16), and the pilots themselves: ``KerasPilot`` / ``ModelType``
@@ -13,13 +13,13 @@ tensor cores.
 from .component import Component  # noqa: F401
 from .config import default_config  # noqa: F401
 
-__all__ = ["Component", "default_config", "ImgPreprocessing", "LocationTracker", "MultiTrackLocationTracker", "SpeedControl", "FrameNormalise",
-           "ControlMultiplexer", "DriverAssistance", "three_segment_map", "KerasPilot", "PilotNet", "ModelType", "native"]
+__all__ = ["Component", "default_config", "ImgPreprocessing", "MultiTrackImgPreprocessing", "LocationTracker", "MultiTrackLocationTracker", "SpeedControl",
+           "FrameNormalise", "ControlMultiplexer", "DriverAssistance", "three_segment_map", "KerasPilot", "PilotNet", "ModelType", "native"]
 
 
 def __getattr__(name):
     # components import torch and load the CUDA library; keep `import triton_racer_sim_b200.synth` light
-    if name in ("ImgPreprocessing", "LocationTracker", "MultiTrackLocationTracker", "SpeedControl", "FrameNormalise", "ControlMultiplexer", "DriverAssistance",
+    if name in ("ImgPreprocessing", "MultiTrackImgPreprocessing", "LocationTracker", "MultiTrackLocationTracker", "SpeedControl", "FrameNormalise", "ControlMultiplexer", "DriverAssistance",
                 "three_segment_map"):
         from . import components
         return getattr(components, name)

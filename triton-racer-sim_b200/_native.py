@@ -11,6 +11,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.environ.get("TRS_B200_LIB") or os.path.join(HERE, "libtrs_b200.so")     # (override: instrumented builds of the same library)
 MAX_HSV = 4
 MAX_TRACKS = 256                                          # TRS_MAX_TRACKS
+MAX_PREPROC_CONFIGS = 16                                  # TRS_MAX_PREPROC_CONFIGS
 STAT_COUNT = 24
 STAT_NAMES = ["frames", "mask0", "mask1", "mask2", "mask3", "edge", "strong", "cand", "hyst_sweeps", "roi_sum",
               "t_wait_frame", "t_strip_walk", "t_phase_a", "t_phase_b", "t_phase_c", "t_total"]
@@ -18,7 +19,7 @@ STAT_NAMES = ["frames", "mask0", "mask1", "mask2", "mask3", "edge", "strong", "c
 # every symbol include/trs_b200.h declares (tests check the library exports exactly these)
 SYMBOLS = [
     "trs_version", "trs_last_error", "trs_kernel_launches", "trs_ctx_create", "trs_ctx_destroy", "trs_ctx_device_info",
-    "trs_set_preproc_params", "trs_preprocess", "trs_normalise", "trs_set_track", "trs_locate", "trs_set_tracks", "trs_locate_tracks", "trs_speed_control",
+    "trs_set_preproc_params", "trs_preprocess", "trs_set_preproc_configs", "trs_preprocess_configs", "trs_normalise", "trs_set_track", "trs_locate", "trs_set_tracks", "trs_locate_tracks", "trs_speed_control",
     "trs_preprocess_host", "trs_host_alloc", "trs_host_free", "trs_debug_canny_stages", "trs_control_mux", "trs_pwm_map",
     "trs_jpeg_decode_host", "trs_telemetry_decode_host", "trs_jpeg_encode", "trs_jpeg_encode_copy",
     "trs_pilot_create", "trs_pilot_destroy", "trs_pilot_forward", "trs_pilot_debug_activation", "trs_pilot_layer_shape",
@@ -86,6 +87,8 @@ def load():
     lib.trs_ctx_device_info.argtypes = [vp] + [C.POINTER(C.c_int)] * 4
     lib.trs_set_preproc_params.argtypes = [vp, C.POINTER(PreprocParams)]
     lib.trs_preprocess.argtypes = [vp, vp, i32, i32, i32, vp, vp, vp, vp]
+    lib.trs_set_preproc_configs.argtypes = [vp, C.POINTER(PreprocParams), i32]
+    lib.trs_preprocess_configs.argtypes = [vp, vp, vp, i32, i32, i32, vp, vp, vp, vp]
     lib.trs_normalise.argtypes = [vp, vp] + [i32] * 9 + [vp, vp, vp]
     lib.trs_set_track.argtypes = [vp, vp, i32, C.c_double, C.c_double]
     lib.trs_locate.argtypes = [vp, vp, i32, vp, vp, vp]

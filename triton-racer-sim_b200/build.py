@@ -7,7 +7,7 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 LIB = os.path.join(HERE, "libtrs_b200.so")
 SOURCES = ["trs_api.cu", "pilot_api.cu"]
-HEADERS = ["pixel_math.cuh", "preproc_kernel.cuh", "preproc_fast.cuh", "preproc_bsw.cuh", "misc_kernels.cuh", "loc_grid.h", "loc_tracks.cuh", "jpeg_core.cuh", "jpeg_host.h", "jpeg_kernels.cuh", "jpeg_enc_core.cuh", "jpeg_enc_kernels.cuh", "pilot_kernels.cuh", "trs_internal.h", os.path.join("..", "..", "include", "trs_b200.h")]
+HEADERS = ["pixel_math.cuh", "preproc_kernel.cuh", "preproc_fast.cuh", "preproc_bsw.cuh", "preproc_list.h", "misc_kernels.cuh", "loc_grid.h", "loc_tracks.cuh", "jpeg_core.cuh", "jpeg_host.h", "jpeg_kernels.cuh", "jpeg_enc_core.cuh", "jpeg_enc_kernels.cuh", "pilot_kernels.cuh", "trs_internal.h", os.path.join("..", "..", "include", "trs_b200.h")]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",   # Blackwell B200 only: no multi-arch fatbin, no PTX fallback
     "-O3", "-lineinfo", "-std=c++17",

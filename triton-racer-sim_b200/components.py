@@ -6,6 +6,7 @@ can be added to the reference's ``Car`` as they are.  All arithmetic runs in the
 ``libtrs_b200.so``; there is no CPU path here.
 
   ImgPreprocessing   components/img_preprocessing.py:9-108       cam/img -> cam/processed_img
+  MultiTrackImgPreprocessing  the same with a configuration per track  cam/img, loc/track -> cam/processed_img
   LocationTracker    components/track_data_process.py:68-107     gym/x, gym/y, gym/z -> loc/segment
   MultiTrackLocationTracker  the same for cars on several tracks    gym/x, gym/y, gym/z, loc/track -> loc/segment
   SpeedControl       components/keras_pilot.py:80-95,99-118,142-153 + utils/mapping.py:23-35
@@ -188,6 +189,118 @@ class ImgPreprocessing(Component):
 
     def getName(self):
         return 'Image Preprocessing'
+
+
+class MultiTrackImgPreprocessing(Component):
+    """``ImgPreprocessing`` for a batch of cars on several tracks: frame i with ``cfgs[t_i]``.
+
+    Each frame's outputs are exactly what ``ImgPreprocessing(cfgs[t_i])`` gives it, in one stream-ordered call for the whole batch.
+    ``cfgs``: one reference config dict per track (its ``myconfig.json``, manage.py:91-94), at most ``nat.MAX_PREPROC_CONFIGS``.
+
+    Inputs ``cam/img, loc/track``; outputs ``cam/processed_img`` [+ ``normalised_key``, the float32 ``/255`` tensor].  ``loc/track`` is the
+    per-car index ``MultiTrackLocationTracker`` takes.  ``step(frames, track)`` accepts
+      * a CUDA uint8 (N,H,W,3) batch with an int32 (N,) CUDA index tensor  -> CUDA tensors      (stream-ordered, no sync)
+      * a numpy uint8 (N,H,W,3) batch with an integer (N,) array           -> numpy             (one upload, one download)
+      * one numpy uint8 (H,W,3) frame with a Python int                    -> numpy (H,W,3)     (N = 1 drop-in)
+      * ``None``                                                            -> ``None``
+    An index outside ``[0, K)`` gives u8 0 and f32 NaN on the device path, and raises ``ValueError`` from the host forms.
+    Calls of one component go to one CUDA stream at a time.
+    """
+
+    def __init__(self, cfgs, device=None, normalised_key=None, collect_stats=False):
+        outputs = ['cam/processed_img'] + ([normalised_key] if normalised_key else [])
+        Component.__init__(self, inputs=['cam/img', 'loc/track'], outputs=outputs, threaded=False)
+        k = len(cfgs)
+        if not 1 <= k <= nat.MAX_PREPROC_CONFIGS:
+            raise ValueError(f"1 to {nat.MAX_PREPROC_CONFIGS} configurations, got {k}")
+        self.cfgs = []
+        for c in cfgs:
+            full = default_config()
+            full.update(c)
+            self.cfgs.append(full)
+        self.n_cfgs = k
+        self.device = _device_index(device)
+        self.ctx = nat.Context(self.device)
+        self.want_f32 = normalised_key is not None
+        self.collect_stats = bool(collect_stats)
+        self._stats_dev = None
+        params = (nat.PreprocParams * k)(*[nat.preproc_params_from_cfg(c) for c in self.cfgs])
+        nat.check(self.ctx.lib.trs_set_preproc_configs(self.ctx.handle, params, k), "trs_set_preproc_configs")
+
+    def process_device(self, frames: torch.Tensor, track: torch.Tensor, out_u8=None, out_f32=None, want_u8=True, want_f32=None):
+        """(N,H,W,3) uint8 and (N,) int32 CUDA tensors -> (u8 tensor or None, f32 tensor or None).  Enqueued on the current stream."""
+        if not isinstance(frames, torch.Tensor) or frames.dtype != torch.uint8 or frames.dim() != 4 or frames.shape[-1] != 3:
+            raise ValueError(f"expected (N,H,W,3) uint8 frames, got {getattr(frames, 'shape', None)} {getattr(frames, 'dtype', type(frames))}")
+        _check_device_tensor(frames, self.device, torch.uint8, "frames")
+        n, h, w, _ = frames.shape
+        _check_device_tensor(track, self.device, torch.int32, "track")
+        if tuple(track.shape) != (n,):
+            raise ValueError(f"track must have shape ({n},), got {tuple(track.shape)}")
+        want_f32 = self.want_f32 if want_f32 is None else want_f32
+        if want_u8 and out_u8 is None:
+            out_u8 = torch.empty_like(frames)
+        if want_f32 and out_f32 is None:
+            out_f32 = torch.empty(frames.shape, dtype=torch.float32, device=frames.device)
+        for t, dt, name in ((out_u8, torch.uint8, "out_u8"), (out_f32, torch.float32, "out_f32")):
+            _check_device_tensor(t, self.device, dt, name)
+            if t is not None and tuple(t.shape) != tuple(frames.shape):
+                raise ValueError(f"{name} must have the frames' shape {tuple(frames.shape)}, got {tuple(t.shape)}")
+        stats = None
+        if self.collect_stats:
+            if self._stats_dev is None:
+                self._stats_dev = torch.zeros((self.n_cfgs, nat.STAT_COUNT), dtype=torch.int64, device=frames.device)
+            self._stats_dev.zero_()
+            stats = self._stats_dev
+        nat.check(self.ctx.lib.trs_preprocess_configs(self.ctx.handle, _ptr(frames), _ptr(track), n, h, w, _ptr(out_u8), _ptr(out_f32),
+                                                      _ptr(stats), _stream_ptr(self.device)), "trs_preprocess_configs")
+        return out_u8, out_f32
+
+    def stats(self) -> list:
+        """Counters of the last device call, one dict per configuration (synchronises)."""
+        if self._stats_dev is None:
+            return []
+        return [dict(zip(nat.STAT_NAMES, row)) for row in self._stats_dev.cpu().tolist()]
+
+    def _host_tracks(self, track, n: int):
+        t = np.asarray(track)
+        if not np.issubdtype(t.dtype, np.integer):
+            raise ValueError(f"track indices must be integers, got {t.dtype}")
+        if t.shape != (n,):
+            raise ValueError(f"track must have shape ({n},), got {t.shape}")
+        if t.size and (t.min() < 0 or t.max() >= self.n_cfgs):
+            raise ValueError(f"track index outside [0, {self.n_cfgs})")
+        return np.ascontiguousarray(t, np.int32)
+
+    def step(self, *args):
+        img, track = args[0], args[1]
+        if img is None:
+            return (None, None) if self.want_f32 else (None,)
+        if isinstance(img, torch.Tensor):
+            u8, f32 = self.process_device(img, track)
+            return (u8, f32) if self.want_f32 else (u8,)
+        arr = np.asarray(img)
+        single = arr.ndim == 3
+        if single:
+            if isinstance(track, (bool, np.bool_)) or not isinstance(track, (int, np.integer)):
+                raise ValueError(f"one frame takes one integer track index, got {type(track).__name__}")
+            track = [track]
+        batch = arr[None] if single else arr
+        if batch.dtype != np.uint8 or batch.ndim != 4 or batch.shape[-1] != 3:
+            raise ValueError(f"expected (N,H,W,3) uint8 frames, got {batch.shape} {batch.dtype}")
+        dev = f"cuda:{self.device}"
+        t = torch.from_numpy(self._host_tracks(track, batch.shape[0])).to(dev)
+        u8, f32 = self.process_device(torch.from_numpy(np.ascontiguousarray(batch)).to(dev), t)
+        u8 = u8.cpu().numpy()
+        f32 = f32.cpu().numpy() if f32 is not None else None
+        if single:
+            u8, f32 = u8[0], (f32[0] if f32 is not None else None)
+        return (u8, f32) if self.want_f32 else (u8,)
+
+    def onShutdown(self):
+        self.ctx.close()
+
+    def getName(self):
+        return 'Multi-Track Image Preprocessing'
 
 
 class LocationTracker(Component):

@@ -155,12 +155,18 @@ __device__ __forceinline__ void p2_nms_lagged(const FastParams& P, const Dims& D
 // frame from exact channel sums over rows 40..118 (img_preprocessing.py:88), read from global memory by the compute warps (the bands read those
 // rows again, from L2); the sums of two consecutive frames alternate between two sets of accumulators, so two barriers among the compute
 // warps per frame are enough.
-template <int NR, int F0, int F1, int H, int W, int R, int NSW = 2, int MAXREG = SW_MAXREG, bool LUT = false>
-__global__ void __maxnreg__(MAXREG) k_preprocess_bsw(const __grid_constant__ FastParams P)
+template <int NR, int F0, int F1, int H, int W, int R, int NSW = 2, int MAXREG = SW_MAXREG, bool LUT = false, bool LIST = false>
+__global__ void __maxnreg__(MAXREG) k_preprocess_bsw(const __grid_constant__ FastParams P, const FrameList fl = {})
 {
     using L = BswLayout<H, W, R, NR, NSW>;
     extern __shared__ __align__(16) uint8_t smem[];
     const PreKParams& p = P.k;
+    int n_list = 0;
+    const int* list = nullptr;
+    if constexpr (LIST) {                                          // (the frame ring holds positions in the list, the loads map them to frames)
+        plist_open(fl, list, n_list);
+        if ((int)blockIdx.x >= n_list) return;
+    }
     uint32_t sb = smem_u32(smem);
     asm volatile("" : "+r"(sb));
     constexpr int NCW = L::NCW, NC = 32 * NCW, NS = 32 * NSW, NT = NC + NS, NB = L::NB, SEG = L::SEG, ww = W / 32, NSLOT = L::NSLOT;
@@ -182,7 +188,7 @@ __global__ void __maxnreg__(MAXREG) k_preprocess_bsw(const __grid_constant__ Fas
     const uint32_t a_stash = sb + L::OFF_STASH, a_zero = a_stash + NCW * 8 * L::STASH_LANE;
     Dims Dm;
     Dm.h = H; Dm.w = W; Dm.mag_stride = W + 4; Dm.plane_bytes = L::MASKP;      // (the walks use plane_bytes for the stride between colour ranges only)
-    const uint32_t n = (uint32_t)p.n;
+    const uint32_t n = (uint32_t)(LIST ? n_list : p.n);
     static_assert(NB >= 2, "the last band reads the next frame after band 0's wait for the hysteresis of the frame before");
 
     uint32_t ticket = 0;
@@ -217,7 +223,7 @@ __global__ void __maxnreg__(MAXREG) k_preprocess_bsw(const __grid_constant__ Fas
         M.store_lane = !(lane & 1);
         const uint32_t my_slot = a_stash + (uint32_t)(warp * 8 + (lane & 7)) * L::STASH_LANE;
         const uint32_t my_bar = bar_p1 + 16 * warp;
-        if (tid == 0 && blockIdx.x < n) issue_band(blockIdx.x, 0);
+        if (tid == 0 && blockIdx.x < n) issue_band(plist_frame<LIST>(list, blockIdx.x), 0);
         uint32_t gb = 0;                                          // bands finished by this warp since the kernel started
         int slot = 0;                                             // gb % NSLOT: the mask slot of the band
         uint32_t round = 0;                                       // gb / NSLOT: how often the slot has been used before
@@ -226,8 +232,9 @@ __global__ void __maxnreg__(MAXREG) k_preprocess_bsw(const __grid_constant__ Fas
         // Frames 0 and 1: set-up barrier.
 #pragma unroll 1
         for (int j = 0;; ++j) {
-            const uint32_t f = ring_frame(a_ring, j);
-            if (f >= n) break;
+            const uint32_t fj = ring_frame(a_ring, j);
+            if (fj >= n) break;
+            const uint32_t f = plist_frame<LIST>(list, fj);
             const uint32_t a_edge = (j & 1) ? S.edge2 : S.edge;
             if (LUT && p.dynamic) {
                 constexpr int Y0 = H < 40 ? H : 40, Y1 = H < 119 ? H : 119, NTRI = (Y1 - Y0) * L::ROWB / 12;      // groups of four pixels = three words
@@ -277,7 +284,7 @@ __global__ void __maxnreg__(MAXREG) k_preprocess_bsw(const __grid_constant__ Fas
                     mbar_arrive(my_bar + 8 * (gb & 1u));
                     if (atom_inc_acq_rel(a_cnt) == (uint32_t)NCW * (gb + 1) - 1) {      // the last warp out: the band's pixels are dead
                         if (b + 1 < NB) issue_band(f, b + 1);
-                        else if (const uint32_t fn = ring_frame(a_ring, j + 1); fn < n) issue_band(fn, 0);
+                        else if (const uint32_t fn = ring_frame(a_ring, j + 1); fn < n) issue_band(plist_frame<LIST>(list, fn), 0);
                     }
                 }
                 // the neighbours' magnitudes of this band (barrier gb & 1 of a warp is in its phase gb >> 1)
@@ -307,8 +314,9 @@ __global__ void __maxnreg__(MAXREG) k_preprocess_bsw(const __grid_constant__ Fas
         // slot j was written by thread NC two frames ago, before a barrier of both store warps
 #pragma unroll 1
         for (int j = 0;; ++j) {
-            const uint32_t f = ring_frame(a_ring, j);
-            if (f >= n) break;
+            const uint32_t fj = ring_frame(a_ring, j);
+            if (fj >= n) break;
+            const uint32_t f = plist_frame<LIST>(list, fj);
             if (st == 0) ticket = draw_frames(p);                 // frame j + 2: published after this frame's hysteresis
             const uint32_t a_edge = (j & 1) ? S.edge2 : S.edge;
             bar_sync(2, NT);

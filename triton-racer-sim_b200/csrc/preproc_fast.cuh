@@ -1181,11 +1181,17 @@ __device__ __forceinline__ void count_planes(const PreKParams& p, const SmemMap&
 // =========================================================================================================
 // Resident kernel: one frame per CTA, two CTAs per SM
 // =========================================================================================================
-template <int NR, bool EDGE, int F0, int F1>
-__global__ void __launch_bounds__(FAST_MAX_THREADS, 2) k_preprocess_fast(const __grid_constant__ FastParams P)
+template <int NR, bool EDGE, int F0, int F1, bool LIST = false>
+__global__ void __launch_bounds__(FAST_MAX_THREADS, 2) k_preprocess_fast(const __grid_constant__ FastParams P, const FrameList fl = {})
 {
     extern __shared__ __align__(16) uint8_t smem[];
     const PreKParams& p = P.k;
+    int n_list = 0;
+    const int* list = nullptr;
+    if constexpr (LIST) {                              // (preproc_kernel.cuh k_preprocess)
+        plist_open(fl, list, n_list);
+        if ((int)blockIdx.x >= n_list) return;
+    }
     const FastGeom& G = P.g;
     uint32_t sb = smem_u32(smem);
     asm volatile("" : "+r"(sb));                       // launder: the window base lives in this register, never re-derived
@@ -1206,7 +1212,7 @@ __global__ void __launch_bounds__(FAST_MAX_THREADS, 2) k_preprocess_fast(const _
     }
     if (tid == 0) { mbar_init(S.bar, 1); asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
     __syncthreads();
-    if (tid == 0 && (int)blockIdx.x < p.n) issue_frame_load(S.pix[0], p.in + (size_t)blockIdx.x * frame_bytes, frame_bytes, S.bar);
+    if (tid == 0 && (int)blockIdx.x < (LIST ? n_list : p.n)) issue_frame_load(S.pix[0], p.in + (size_t)plist_frame<LIST>(list, blockIdx.x) * frame_bytes, frame_bytes, S.bar);
     uint32_t phase = 0;
     uint32_t pa[3];
     plane_sources(p, S.edge, S.mask, G.plane_bytes, pa);
@@ -1219,7 +1225,8 @@ __global__ void __launch_bounds__(FAST_MAX_THREADS, 2) k_preprocess_fast(const _
 #else
     const bool timing = false;
 #endif
-    for (int f = blockIdx.x; f < p.n; f += gridDim.x) {
+    for (int j = blockIdx.x; j < (LIST ? n_list : p.n); j += gridDim.x) {
+        const int f = plist_frame<LIST>(list, j);
         const long long tk0 = timing ? clock64() : 0;
         mbar_wait(S.bar, phase);
         phase ^= 1u;
@@ -1228,8 +1235,8 @@ __global__ void __launch_bounds__(FAST_MAX_THREADS, 2) k_preprocess_fast(const _
         p1_strip_walk<NR, EDGE, F0, F1>(P, Dm, S.pix[0], S.mag[0], S.mask, S, M, G.seg_rows_front);
         __syncthreads();
         const long long tk2 = timing ? clock64() : 0;
-        if (!p.need_pixels && tid == 0 && f + (int)gridDim.x < p.n)       // pixels are dead: prefetch the next frame
-            issue_frame_load(S.pix[0], p.in + (size_t)(f + gridDim.x) * frame_bytes, frame_bytes, S.bar);
+        if (!p.need_pixels && tid == 0 && j + (int)gridDim.x < (LIST ? n_list : p.n))         // pixels are dead: prefetch the next frame
+            issue_frame_load(S.pix[0], p.in + (size_t)plist_frame<LIST>(list, j + gridDim.x) * frame_bytes, frame_bytes, S.bar);
         long long tk3 = tk2, tk4 = tk2;
         if (EDGE) {
             p2_nms(P, Dm, S.mag[0], S.cand, S.edge, S, M, G.seg_rows_front);
@@ -1247,8 +1254,8 @@ __global__ void __launch_bounds__(FAST_MAX_THREADS, 2) k_preprocess_fast(const _
             const long long tk5 = clock64();
             tm[0] += tk1 - tk0; tm[1] += tk2 - tk1; tm[2] += tk3 - tk2; tm[3] += tk4 - tk3; tm[4] += tk5 - tk4; tm[5] += tk5 - tk0;
         }
-        if (p.need_pixels && tid == 0 && f + (int)gridDim.x < p.n)
-            issue_frame_load(S.pix[0], p.in + (size_t)(f + gridDim.x) * frame_bytes, frame_bytes, S.bar);
+        if (p.need_pixels && tid == 0 && j + (int)gridDim.x < (LIST ? n_list : p.n))
+            issue_frame_load(S.pix[0], p.in + (size_t)plist_frame<LIST>(list, j + gridDim.x) * frame_bytes, frame_bytes, S.bar);
     }
     if (timing) {
 #pragma unroll
@@ -1297,11 +1304,17 @@ __device__ __forceinline__ float dynamic_delta_global(const PreKParams& p, const
 // they land (the dynamic one is built first from the frame's rows 40..118 in global memory); an output channel that keeps the adjusted pixel
 // reads the frame again in the output phase (from L2: 296 frames in flight are 68 MB).
 // =========================================================================================================
-template <int NR, bool EDGE, int F0, int F1>
-__global__ void __launch_bounds__(FAST_MAX_THREADS, 2) k_preprocess_banded(const __grid_constant__ FastParams P)
+template <int NR, bool EDGE, int F0, int F1, bool LIST = false>
+__global__ void __launch_bounds__(FAST_MAX_THREADS, 2) k_preprocess_banded(const __grid_constant__ FastParams P, const FrameList fl = {})
 {
     extern __shared__ __align__(16) uint8_t smem[];
     const PreKParams& p = P.k;
+    int n_list = 0;
+    const int* list = nullptr;
+    if constexpr (LIST) {
+        plist_open(fl, list, n_list);
+        if ((int)blockIdx.x >= n_list) return;
+    }
     const FastGeom& G = P.g;
     uint32_t sb = smem_u32(smem);
     asm volatile("" : "+r"(sb));
@@ -1326,14 +1339,15 @@ __global__ void __launch_bounds__(FAST_MAX_THREADS, 2) k_preprocess_banded(const
         const int p0 = max(b * BH - 2, 0), p1 = min(min((b + 1) * BH, h) + 2, h);
         issue_frame_load(S.pix[0], p.in + f * frame_bytes + (size_t)p0 * row_bytes, (uint32_t)(p1 - p0) * row_bytes, S.bar);
     };
-    if (tid == 0 && (int)blockIdx.x < p.n) issue_band(blockIdx.x, 0);
+    if (tid == 0 && (int)blockIdx.x < (LIST ? n_list : p.n)) issue_band(plist_frame<LIST>(list, blockIdx.x), 0);
 
     uint32_t phase = 0;
     uint32_t pa[3];
     plane_sources(p, S.edge, S.mask, G.plane_bytes, pa);
     unsigned long long* s_red = reinterpret_cast<unsigned long long*>(smem + G.off_red);
     const bool use_lut = p.dynamic || !p.lut_identity;
-    for (int f = blockIdx.x; f < p.n; f += gridDim.x) {
+    for (int j = blockIdx.x; j < (LIST ? n_list : p.n); j += gridDim.x) {
+        const int f = plist_frame<LIST>(list, j);
         if (p.dynamic) {
             // the brightness statistic covers rows 40..118 (img_preprocessing.py:88), which no single band holds: exact channel sums from the
             // frame in global memory while the first band's copy is in flight (the bands read those rows again, from L2), then this frame's table
@@ -1366,7 +1380,8 @@ __global__ void __launch_bounds__(FAST_MAX_THREADS, 2) k_preprocess_banded(const
             __syncthreads();
             if (tid == 0) {                                         // pixels are dead: fetch the next band (of this or the next frame)
                 if (b + 1 < NB) issue_band(f, b + 1);
-                else if (f + (int)gridDim.x < p.n) issue_band((size_t)f + gridDim.x, 0);
+                else if (j + (int)gridDim.x < (LIST ? n_list : p.n))
+                    issue_band(LIST ? (size_t)plist_frame<LIST>(list, j + gridDim.x) : (size_t)f + gridDim.x, 0);
             }
             if (EDGE) {
                 const StripMap M2 = strip_map(warp, lane, ww, G.seg_rows_nms, by1, by0);
@@ -1434,11 +1449,17 @@ inline bool sw_static_geometry_ok(const FastGeom& g, int h, int w)
            sw_seg_rows<H, W>() % 3 == 0 && 4 * ((SW_COMPUTE_THREADS / 32) / (W / 32)) * sw_seg_rows<H, W>() == H;      // the segments tile the rows exactly
 }
 
-template <int NR, int F0, int F1, int H = 0, int W = 0>
-__global__ void __maxnreg__(SW_MAXREG) k_preprocess_sw(const __grid_constant__ FastParams P)
+template <int NR, int F0, int F1, int H = 0, int W = 0, bool LIST = false>
+__global__ void __maxnreg__(SW_MAXREG) k_preprocess_sw(const __grid_constant__ FastParams P, const FrameList fl = {})
 {
     extern __shared__ __align__(16) uint8_t smem[];
     const PreKParams& p = P.k;
+    int n_list = 0;
+    const int* list = nullptr;
+    if constexpr (LIST) {                                          // (the frame ring holds positions in the list, the loads map them to frames)
+        plist_open(fl, list, n_list);
+        if ((int)blockIdx.x >= n_list) return;
+    }
     const FastGeom& G = P.g;
     uint32_t sb = smem_u32(smem);
     asm volatile("" : "+r"(sb));
@@ -1454,7 +1475,7 @@ __global__ void __maxnreg__(SW_MAXREG) k_preprocess_sw(const __grid_constant__ F
     const uint32_t frame_bytes = (uint32_t)h * w * 3;
     const int plane_words = h * ww;
     const int NC = SW_COMPUTE_THREADS;
-    const uint32_t n = (uint32_t)p.n;
+    const uint32_t n = (uint32_t)(LIST ? n_list : p.n);
     const uint32_t mask_set_bytes = (uint32_t)(NR * Dm.plane_bytes);
     const uint32_t main_bytes = frame_bytes - (uint32_t)tail_bytes;
     const uint32_t bar_main = S.bar, bar_tail = S.bar + 8, bar_free = S.bar + 16;      // bar_free + 8 q: plane set q has been written out
@@ -1484,7 +1505,7 @@ __global__ void __maxnreg__(SW_MAXREG) k_preprocess_sw(const __grid_constant__ F
         int tail_k = tail_row - (nsegs - 1) * seg_rows + 1;
         tail_k = tail_k < 0 ? 0 : (tail_k / 3) * 3;
         if (tid == 0 && blockIdx.x < n) {
-            const uint8_t* src = p.in + (size_t)blockIdx.x * frame_bytes;
+            const uint8_t* src = p.in + (size_t)plist_frame<LIST>(list, blockIdx.x) * frame_bytes;
             issue_frame_piece(S.pix[0], src, 0, main_bytes, bar_main);
             if (tail_bytes) issue_frame_piece(S.pix[0], src, main_bytes, frame_bytes, bar_tail);
         }
@@ -1516,7 +1537,7 @@ __global__ void __maxnreg__(SW_MAXREG) k_preprocess_sw(const __grid_constant__ F
             TRS_TICK(tk4);
             if (tid == 0) {                                              // pixels are dead: prefetch the next frame (all but its tail)
                 const uint32_t fn = ring_frame(a_ring, j + 1);
-                if (fn < n) issue_frame_piece(S.pix[0], p.in + (size_t)fn * frame_bytes, 0, main_bytes, bar_main);
+                if (fn < n) issue_frame_piece(S.pix[0], p.in + (size_t)plist_frame<LIST>(list, fn) * frame_bytes, 0, main_bytes, bar_main);
             }
             p2_nms<(STATIC ? sw_seg_rows<(STATIC ? H : 32), (STATIC ? W : 32)>() : 0), false>(P, Dm, S.mag[0], S.cand, a_edge, S, M, seg_rows);
             bar_sync(1, NC);
@@ -1542,8 +1563,9 @@ __global__ void __maxnreg__(SW_MAXREG) k_preprocess_sw(const __grid_constant__ F
         // ------------------------------------------------ store warps -------------------------------------------------
         // slots j and j + 1 were written by thread NC at least two frames ago, before a barrier of both store warps
         for (int j = 0;; ++j) {
-            const uint32_t f = ring_frame(a_ring, j);
-            if (f >= n) break;
+            const uint32_t fj = ring_frame(a_ring, j);
+            if (fj >= n) break;
+            const uint32_t f = plist_frame<LIST>(list, fj);
             if (tid == NC) ticket = draw_frames(p);                      // frame j + 3: published after this frame's output
             uint32_t pa[3];
             plane_sources(p, (j & 1) ? S.edge2 : S.edge, S.mask + (j & 1) * mask_set_bytes, Dm.plane_bytes, pa);
@@ -1563,7 +1585,7 @@ __global__ void __maxnreg__(SW_MAXREG) k_preprocess_sw(const __grid_constant__ F
                 }
                 if (tid == NC && tail_bytes) {                           // the candidate plane is dead: fetch the tail it was sitting in
                     const uint32_t fn = ring_frame(a_ring, j + 1);
-                    if (fn < n) issue_frame_piece(S.pix[0], p.in + (size_t)fn * frame_bytes, main_bytes, frame_bytes, bar_tail);
+                    if (fn < n) issue_frame_piece(S.pix[0], p.in + (size_t)plist_frame<LIST>(list, fn) * frame_bytes, main_bytes, frame_bytes, bar_tail);
                 }
             }
             p4_output(P, Dm, pa, S.pix[0], p.out_u8 ? p.out_u8 + (size_t)f * frame_bytes : nullptr, p.out_f32 ? p.out_f32 + (size_t)f * frame_bytes : nullptr,
@@ -1586,8 +1608,15 @@ __global__ void __maxnreg__(SW_MAXREG) k_preprocess_sw(const __grid_constant__ F
 // Frame bytes and row bytes must be multiples of 4.
 // =========================================================================================================
 enum { ADJ_THREADS = 256 };
-__global__ void __launch_bounds__(ADJ_THREADS) k_adjust_stream(const __grid_constant__ PreKParams p)
+template <bool LIST = false>
+__global__ void __launch_bounds__(ADJ_THREADS) k_adjust_stream(const __grid_constant__ PreKParams p, const FrameList fl = {})
 {
+    int n_list = 0;
+    const int* list = nullptr;
+    if constexpr (LIST) {
+        plist_open(fl, list, n_list);
+        if ((int)blockIdx.x >= n_list) return;
+    }
     __shared__ __align__(16) uint8_t s_lut[256];
     __shared__ unsigned long long s_red[4 + 16];
     const int tid = threadIdx.x, nthr = blockDim.x, lane = tid & 31;
@@ -1599,7 +1628,8 @@ __global__ void __launch_bounds__(ADJ_THREADS) k_adjust_stream(const __grid_cons
     for (int i = tid; i < 256; i += nthr) s_lut[i] = p.lut[i];
     for (int i = tid; i < 4 + 16; i += nthr) s_red[i] = 0;
     __syncthreads();
-    for (int f = blockIdx.x; f < p.n; f += gridDim.x) {
+    for (int j = blockIdx.x; j < (LIST ? n_list : p.n); j += gridDim.x) {
+        const int f = plist_frame<LIST>(list, j);
         const uint8_t* gfr = p.in + (size_t)f * frame_bytes;
         if (p.dynamic) {
             const float fdelta = dynamic_delta_global(p, gfr, s_red, tid, nthr, lane);
@@ -1629,7 +1659,7 @@ __global__ void __launch_bounds__(ADJ_THREADS) k_adjust_stream(const __grid_cons
     if (p.stats) {
         __syncthreads();
         if (tid == 0) {
-            const int mine = (int)blockIdx.x < p.n ? (p.n - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x : 0;
+            const int mine = (int)blockIdx.x < (LIST ? n_list : p.n) ? ((LIST ? n_list : p.n) - (int)blockIdx.x + (int)gridDim.x - 1) / (int)gridDim.x : 0;
             if (mine) atomicAdd(&p.stats[0], (unsigned long long)mine);
             if (s_red[4 + 9]) atomicAdd(&p.stats[9], s_red[4 + 9]);
         }

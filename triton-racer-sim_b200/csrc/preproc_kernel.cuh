@@ -19,6 +19,7 @@
 #include <stdint.h>
 
 #include "pixel_math.cuh"
+#include "preproc_list.h"
 
 namespace trs {
 
@@ -94,8 +95,17 @@ __device__ __forceinline__ uint32_t lut4(const uint8_t* lut, uint32_t v)
            ((uint32_t)lut[v >> 24] << 24);
 }
 
-__global__ void __launch_bounds__(PRE_THREADS, 1) k_preprocess(const __grid_constant__ PreKParams p)
+// LIST (trs_preprocess_configs): the launch works on the frames of one bucket (preproc_list.h), the frame count read from fl; the CTAs
+// without a first frame leave at once.
+template <bool LIST = false>
+__global__ void __launch_bounds__(PRE_THREADS, 1) k_preprocess(const __grid_constant__ PreKParams p, const FrameList fl = {})
 {
+    int n_list = 0;
+    const int* list = nullptr;
+    if constexpr (LIST) {
+        plist_open(fl, list, n_list);
+        if ((int)blockIdx.x >= n_list) return;
+    }
     extern __shared__ __align__(16) uint8_t smem[];
     const PreSmemLayout L = pre_smem_layout(p.h, p.w, p.band_h, p.row_stride, p.mag_stride, p.wwords, p.n_ranges);
     uint8_t* s_pix = smem + L.pix_off;
@@ -126,7 +136,8 @@ __global__ void __launch_bounds__(PRE_THREADS, 1) k_preprocess(const __grid_cons
     unsigned long long st_edge = 0, st_strong = 0, st_cand = 0, st_sweeps = 0, st_roi = 0, st_frames = 0;
     __syncthreads();
 
-    for (int f = blockIdx.x; f < p.n; f += gridDim.x) {
+    for (int j = blockIdx.x; j < (LIST ? n_list : p.n); j += gridDim.x) {
+        const int f = LIST ? list[j] : j;
         const uint8_t* __restrict__ gin = p.in + (size_t)f * frame_bytes;
 
         // ---- dynamic brightness: ROI sums (rows 40..118) -> per-frame table -------------------------------
@@ -384,6 +395,24 @@ __global__ void __launch_bounds__(PRE_THREADS, 1) k_preprocess(const __grid_cons
             unsigned long long x = v[k];
             for (int o = 16; o; o >>= 1) x += __shfl_xor_sync(0xffffffffu, x, o);
             if (lane == 0 && x) atomicAdd(&p.stats[k], x);
+        }
+    }
+}
+
+// trs_preprocess_configs: the frames of bucket fl.cfg = K, whose configuration index is outside [0, K), get u8 0 and f32 NaN (the -1 / NaN of
+// trs_locate_tracks' out-of-range cars), a CTA per frame at a time.
+enum { UNCFG_THREADS = 256 };
+__global__ void __launch_bounds__(UNCFG_THREADS) k_preprocess_unconfigured(const FrameList fl, size_t frame_bytes, uint8_t* __restrict__ out_u8,
+                                                                          float* __restrict__ out_f32)
+{
+    const int* list;
+    int n;
+    plist_open(fl, list, n);
+    for (int j = blockIdx.x; j < n; j += gridDim.x) {
+        const size_t base = (size_t)list[j] * frame_bytes;
+        for (size_t i = threadIdx.x; i < frame_bytes; i += UNCFG_THREADS) {
+            if (out_u8) out_u8[base + i] = 0;
+            if (out_f32) out_f32[base + i] = __int_as_float(0x7fc00000);
         }
     }
 }

@@ -106,6 +106,13 @@ struct trs_ctx {
     size_t tk_smem = 0;                // the largest grid table (dynamic shared memory of k_locate_tracks_grid)
     int* tk_scratch = nullptr;         // [0] list count | bucket starts (K + 2) | counts ((K + 1) x blocks) | bucketed cars (N) | list (N)
     size_t tk_scratch_cap = 0;         // ints
+    // several preprocessing configurations (trs_set_preproc_configs / trs_preprocess_configs): the derived sets, a frame counter per
+    // configuration, and the bucketing scratch: [0] unused count | bucket starts (K + 2) | counts ((K + 1) x blocks) | bucketed frames (N)
+    int n_cfgs = 0;
+    std::vector<trs::PreKParams> cfg_kp;
+    uint32_t* cfg_ctr = nullptr;
+    int* cfg_scratch = nullptr;
+    size_t cfg_scratch_cap = 0;        // ints
     // host pipeline
     cudaStream_t hs[HOST_STREAMS] = {nullptr, nullptr, nullptr};
     uint8_t* st_in[HOST_STREAMS] = {nullptr, nullptr, nullptr};
@@ -153,9 +160,10 @@ void default_params(trs_preproc_params* p)
     p->canny_b = 100;
 }
 
-int derive_params(trs_ctx* ctx, const trs_preproc_params* u)
+// validation and derivation of one configuration into k (geometry and pointers are filled per call)
+int derive_kparams(const trs_preproc_params* u, trs::PreKParams& k)
 {
-    trs::PreKParams k{};
+    k = trs::PreKParams{};
     if (u->color_filter_enabled && (u->n_hsv < 0 || u->n_hsv > TRS_MAX_HSV))
         return fail(TRS_E_ARG, "n_hsv=%d outside [0,%d]", u->n_hsv, TRS_MAX_HSV);
     // brightness / contrast (img_preprocessing.py:81-102)
@@ -210,6 +218,13 @@ int derive_params(trs_ctx* ctx, const trs_preproc_params* u)
     if (!(a > -2e9 && b < 2e9)) return fail(TRS_E_ARG, "edge thresholds out of range");
     k.low = (int)floor(a);
     k.high = (int)floor(b);
+    return 0;
+}
+
+int derive_params(trs_ctx* ctx, const trs_preproc_params* u)
+{
+    trs::PreKParams k;
+    if (const int rc = derive_kparams(u, k)) return rc;
     ctx->kp = k;
     ctx->user = *u;
     ctx->have_params = true;
@@ -245,34 +260,40 @@ int plan_geometry(trs_ctx* ctx, int h, int w, int n_ranges, Geometry* g)
 
 // Frame-resident fast path (preproc_fast.cuh): whole frame + magnitude plane + bit planes in one CTA's shared memory,
 // width a multiple of 32, everything 16-byte aligned.  Returns 1 if launched, 0 if not eligible, <0 / >1 on error.
+// fl: null for a whole batch; otherwise the list-mode instantiation over one configuration's frames (its frame counter was zeroed by the caller)
 template <int NR, bool EDGE, int F0, int F1>
-int launch_fast_tf(const trs::FastParams& fp, int grid, cudaStream_t st)
+int launch_fast_tf(const trs::FastParams& fp, int grid, cudaStream_t st, const trs::FrameList* fl)
 {
+    const trs::FrameList L = fl ? *fl : trs::FrameList{};
     if (EDGE && fp.use_store_warp) {
         // the reference's camera size with its default colour ranges (core/config.py:8-9,23) gets the variant with compile-time dimensions
-        cudaError_t e = cudaMemsetAsync(fp.k.frame_ctr, 0, sizeof(uint32_t), st);      // the launch's frame tickets start at 0
+        cudaError_t e = fl ? cudaSuccess : cudaMemsetAsync(fp.k.frame_ctr, 0, sizeof(uint32_t), st);      // the launch's frame tickets start at 0
         if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(frame counter)");
         if (NR == 2 && F0 >= 0 && trs::sw_static_geometry_ok<120, 160>(fp.g, fp.k.h, fp.k.w)) {
-            auto kern = trs::k_preprocess_sw<NR, F0, F1, (NR == 2 && F0 >= 0 ? 120 : 0), (NR == 2 && F0 >= 0 ? 160 : 0)>;
+            auto kern = fl ? trs::k_preprocess_sw<NR, F0, F1, (NR == 2 && F0 >= 0 ? 120 : 0), (NR == 2 && F0 >= 0 ? 160 : 0), true>
+                           : trs::k_preprocess_sw<NR, F0, F1, (NR == 2 && F0 >= 0 ? 120 : 0), (NR == 2 && F0 >= 0 ? 160 : 0)>;
             e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, fp.g.total);
             if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(sw 120x160)");
-            kern<<<grid, trs::SW_THREADS, fp.g.total, st>>>(fp);
+            kern<<<grid, trs::SW_THREADS, fp.g.total, st>>>(fp, L);
             return 0;
         }
-        e = cudaFuncSetAttribute(trs::k_preprocess_sw<NR, F0, F1>, cudaFuncAttributeMaxDynamicSharedMemorySize, fp.g.total);
+        auto kern = fl ? trs::k_preprocess_sw<NR, F0, F1, 0, 0, true> : trs::k_preprocess_sw<NR, F0, F1>;
+        e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, fp.g.total);
         if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(sw)");
-        trs::k_preprocess_sw<NR, F0, F1><<<grid, trs::SW_THREADS, fp.g.total, st>>>(fp);
+        kern<<<grid, trs::SW_THREADS, fp.g.total, st>>>(fp, L);
         return 0;
     }
     if (fp.g.n_bands > 1) {
-        cudaError_t e = cudaFuncSetAttribute(trs::k_preprocess_banded<NR, EDGE, F0, F1>, cudaFuncAttributeMaxDynamicSharedMemorySize, fp.g.total);
+        auto kern = fl ? trs::k_preprocess_banded<NR, EDGE, F0, F1, true> : trs::k_preprocess_banded<NR, EDGE, F0, F1>;
+        cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, fp.g.total);
         if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(banded)");
-        trs::k_preprocess_banded<NR, EDGE, F0, F1><<<grid, fp.g.threads, fp.g.total, st>>>(fp);
+        kern<<<grid, fp.g.threads, fp.g.total, st>>>(fp, L);
         return 0;
     }
-    cudaError_t e = cudaFuncSetAttribute(trs::k_preprocess_fast<NR, EDGE, F0, F1>, cudaFuncAttributeMaxDynamicSharedMemorySize, fp.g.total);
+    auto kern = fl ? trs::k_preprocess_fast<NR, EDGE, F0, F1, true> : trs::k_preprocess_fast<NR, EDGE, F0, F1>;
+    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, fp.g.total);
     if (e != cudaSuccess) return cuda_fail(e, "cudaFuncSetAttribute(fast)");
-    trs::k_preprocess_fast<NR, EDGE, F0, F1><<<grid, fp.g.threads, fp.g.total, st>>>(fp);
+    kern<<<grid, fp.g.threads, fp.g.total, st>>>(fp, L);
     return 0;
 }
 
@@ -281,22 +302,23 @@ int launch_fast_tf(const trs::FastParams& fp, int grid, cudaStream_t st)
 enum { DEFAULT_F0 = 8 | 16, DEFAULT_F1 = 1 | 2 | 4 | 16 };
 
 template <int NR, bool EDGE>
-int launch_fast_t(const trs::FastParams& fp, int grid, cudaStream_t st)
+int launch_fast_t(const trs::FastParams& fp, int grid, cudaStream_t st, const trs::FrameList* fl)
 {
     // (the baked variant turns the hue bounds of range 1 into per-delta numerator thresholds and skips the blue-max hue formula, which
     // needs an upper bound below 60: preproc_fast.cuh HueThresholds / hsv_masks_of)
     if (NR == 2 && fp.fr[0].flags == DEFAULT_F0 && fp.fr[1].flags == DEFAULT_F1 && fp.k.ranges[1].hi[0] <= 59)
-        return launch_fast_tf<NR, EDGE, (NR == 2 ? (int)DEFAULT_F0 : -1), (NR == 2 ? (int)DEFAULT_F1 : -1)>(fp, grid, st);
-    return launch_fast_tf<NR, EDGE, -1, -1>(fp, grid, st);
+        return launch_fast_tf<NR, EDGE, (NR == 2 ? (int)DEFAULT_F0 : -1), (NR == 2 ? (int)DEFAULT_F1 : -1)>(fp, grid, st, fl);
+    return launch_fast_tf<NR, EDGE, -1, -1>(fp, grid, st, fl);
 }
 
 // Banded store-warp kernel (preproc_bsw.cuh) for one compile-time geometry.  Returns 1 if launched, 0 if it does not fit, < 0 on error.
 // LUT: a brightness / contrast table that is not the identity.
 template <int H, int W, int R, int NSW, int MAXREG = trs::SW_MAXREG, bool LUT = false>
-int launch_bsw(trs_ctx* ctx, const trs::FastParams& fp, int n, cudaStream_t st)
+int launch_bsw(trs_ctx* ctx, const trs::FastParams& fp, int n, cudaStream_t st, const trs::FrameList* fl)
 {
     using L = trs::BswLayout<H, W, R, 2, NSW>;
-    auto kern = trs::k_preprocess_bsw<2, (int)DEFAULT_F0, (int)DEFAULT_F1, H, W, R, NSW, MAXREG, LUT>;
+    auto kern = fl ? trs::k_preprocess_bsw<2, (int)DEFAULT_F0, (int)DEFAULT_F1, H, W, R, NSW, MAXREG, LUT, true>
+                   : trs::k_preprocess_bsw<2, (int)DEFAULT_F0, (int)DEFAULT_F1, H, W, R, NSW, MAXREG, LUT>;
     if (L::TOTAL > (ctx->smem_optin + 1024) / 2 - 1024) return 0;
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, L::TOTAL);
     if (e != cudaSuccess) { cuda_fail(e, "cudaFuncSetAttribute(bsw)"); return -100 - (int)e; }
@@ -306,16 +328,17 @@ int launch_bsw(trs_ctx* ctx, const trs::FastParams& fp, int n, cudaStream_t st)
     if (per_sm < 1) return 0;
     int grid = ctx->sm_count * per_sm;
     if (grid > n) grid = n;
-    e = cudaMemsetAsync(fp.k.frame_ctr, 0, sizeof(uint32_t), st);                  // the launch's frame tickets start at 0
+    e = fl ? cudaSuccess : cudaMemsetAsync(fp.k.frame_ctr, 0, sizeof(uint32_t), st);      // the launch's frame tickets start at 0
     if (e != cudaSuccess) { cuda_fail(e, "cudaMemsetAsync(frame counter)"); return -100 - (int)e; }
-    kern<<<grid, L::THREADS, L::TOTAL, st>>>(fp);
+    kern<<<grid, L::THREADS, L::TOTAL, st>>>(fp, fl ? *fl : trs::FrameList{});
     g_launches.fetch_add(1, std::memory_order_relaxed);
     e = cudaGetLastError();
     if (e != cudaSuccess) { cuda_fail(e, "k_preprocess_bsw launch"); return -100 - (int)e; }
     return 1;
 }
 
-int try_launch_fast(trs_ctx* ctx, const trs::PreKParams& k, int n, int h, int w, cudaStream_t st)
+// fl: null for the whole batch of n frames; otherwise one configuration's frames out of a batch of n (the grid is sized for n)
+int try_launch_fast(trs_ctx* ctx, const trs::PreKParams& k, int n, int h, int w, cudaStream_t st, const trs::FrameList* fl)
 {
     if (ctx->sw.force_generic) return 0;
     if (!k.edge_enabled && k.n_ranges == 0) {
@@ -323,7 +346,8 @@ int try_launch_fast(trs_ctx* ctx, const trs::PreKParams& k, int n, int h, int w,
         if (!k.word_io || ctx->sw.no_banded) return 0;
         int grid = ctx->sm_count * 8;
         if (grid > n) grid = n;
-        trs::k_adjust_stream<<<grid, trs::ADJ_THREADS, 0, st>>>(k);
+        if (fl) trs::k_adjust_stream<true><<<grid, trs::ADJ_THREADS, 0, st>>>(k, *fl);
+        else trs::k_adjust_stream<<<grid, trs::ADJ_THREADS, 0, st>>>(k);
         g_launches.fetch_add(1, std::memory_order_relaxed);
         cudaError_t e = cudaGetLastError();
         if (e != cudaSuccess) { cuda_fail(e, "k_adjust_stream launch"); return -100 - (int)e; }
@@ -398,16 +422,16 @@ int try_launch_fast(trs_ctx* ctx, const trs::PreKParams& k, int n, int h, int w,
     const bool bsw_ok = k.n_ranges == 2 && k.edge_enabled && !k.need_pixels && !ctx->sw.no_store_warp &&
                         fp.fr[0].flags == DEFAULT_F0 && fp.fr[1].flags == DEFAULT_F1 && k.ranges[1].hi[0] <= 59;
     if (bsw_ok && h == 240 && w == 320) {
-        rc = (k.dynamic || !k.lut_identity) ? launch_bsw<240, 320, 24, 2, trs::SW_MAXREG, true>(ctx, fp, n, st) : launch_bsw<240, 320, 24, 2>(ctx, fp, n, st);
+        rc = (k.dynamic || !k.lut_identity) ? launch_bsw<240, 320, 24, 2, trs::SW_MAXREG, true>(ctx, fp, n, st, fl) : launch_bsw<240, 320, 24, 2>(ctx, fp, n, st, fl);
         if (rc) return rc;
     }
     switch (k.n_ranges * 2 + (k.edge_enabled ? 1 : 0)) {
-    case 1: rc = launch_fast_t<0, true>(fp, grid, st); break;
-    case 2: rc = launch_fast_t<1, false>(fp, grid, st); break;
-    case 3: rc = launch_fast_t<1, true>(fp, grid, st); break;
-    case 4: rc = launch_fast_t<2, false>(fp, grid, st); break;
-    case 5: rc = launch_fast_t<2, true>(fp, grid, st); break;
-    case 6: rc = launch_fast_t<3, false>(fp, grid, st); break;
+    case 1: rc = launch_fast_t<0, true>(fp, grid, st, fl); break;
+    case 2: rc = launch_fast_t<1, false>(fp, grid, st, fl); break;
+    case 3: rc = launch_fast_t<1, true>(fp, grid, st, fl); break;
+    case 4: rc = launch_fast_t<2, false>(fp, grid, st, fl); break;
+    case 5: rc = launch_fast_t<2, true>(fp, grid, st, fl); break;
+    case 6: rc = launch_fast_t<3, false>(fp, grid, st, fl); break;
     default: return 0;
     }
     if (rc) return rc < 0 ? rc : -100 - rc;
@@ -417,20 +441,23 @@ int try_launch_fast(trs_ctx* ctx, const trs::PreKParams& k, int n, int h, int w,
     return 1;
 }
 
-// ctr_slot: the context's frame counter this launch may use (trs_ctx::frame_ctr): launches that can overlap on the device take different slots
+// ctr_slot: the context's frame counter this launch may use (trs_ctx::frame_ctr): launches that can overlap on the device take different slots.
+// fl / kp (trs_preprocess_configs): one configuration's frames out of the batch of n, with that configuration's derived parameters and frame
+// counter in kp; both null: the whole batch with the context's configuration.
 int launch_preprocess(trs_ctx* ctx, const uint8_t* in, int n, int h, int w, uint8_t* out_u8, float* out_f32,
-                      unsigned long long* stats, uint16_t* dbg_mag, uint8_t* dbg_map, bool force_edge, cudaStream_t st, int ctr_slot)
+                      unsigned long long* stats, uint16_t* dbg_mag, uint8_t* dbg_map, bool force_edge, cudaStream_t st, int ctr_slot,
+                      const trs::FrameList* fl = nullptr, const trs::PreKParams* kp = nullptr)
 {
-    trs::PreKParams k = ctx->kp;
+    trs::PreKParams k = kp ? *kp : ctx->kp;
     if (force_edge && !k.edge_enabled) { k.edge_enabled = 1; }
     if (!dbg_mag && !dbg_map) {
         trs::PreKParams kf = k;
         kf.in = in; kf.out_u8 = out_u8; kf.out_f32 = out_f32; kf.stats = stats; kf.dbg_mag = nullptr; kf.dbg_map = nullptr;
-        kf.frame_ctr = ctx->frame_ctr + ctr_slot;
+        kf.frame_ctr = kp ? kp->frame_ctr : ctx->frame_ctr + ctr_slot;
         kf.n = n; kf.h = h; kf.w = w;
         kf.word_io = ((w * 3) % 4 == 0) && (((uintptr_t)in & 15) == 0) && (!out_u8 || ((uintptr_t)out_u8 & 15) == 0) &&
                      (!out_f32 || ((uintptr_t)out_f32 & 15) == 0) && (((size_t)h * w * 3) % 4 == 0);
-        const int fr = try_launch_fast(ctx, kf, n, h, w, st);
+        const int fr = try_launch_fast(ctx, kf, n, h, w, st, fl);
         if (fr == 1) return 0;
         if (fr < 0) return fr <= -100 ? -(fr + 100) : fr;
     }
@@ -443,13 +470,14 @@ int launch_preprocess(trs_ctx* ctx, const uint8_t* in, int n, int h, int w, uint
     const size_t frame_bytes = (size_t)h * w * 3;
     k.word_io = ((w * 3) % 4 == 0) && (((uintptr_t)in & 15) == 0) && (!out_u8 || ((uintptr_t)out_u8 & 15) == 0) &&
                 (!out_f32 || ((uintptr_t)out_f32 & 15) == 0) && (frame_bytes % 4 == 0);
-    CU(cudaFuncSetAttribute(trs::k_preprocess, cudaFuncAttributeMaxDynamicSharedMemorySize, g.smem));
+    auto kern = fl ? trs::k_preprocess<true> : trs::k_preprocess<false>;
+    CU(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, g.smem));
     int per_sm = 0;
-    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, trs::k_preprocess, trs::PRE_THREADS, g.smem));
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, trs::PRE_THREADS, g.smem));
     if (per_sm < 1) return fail(TRS_E_RANGE, "kernel does not fit an SM with %d B shared memory", g.smem);
     int grid = ctx->sm_count * per_sm;
     if (grid > n) grid = n;
-    trs::k_preprocess<<<grid, trs::PRE_THREADS, g.smem, st>>>(k);
+    kern<<<grid, trs::PRE_THREADS, g.smem, st>>>(k, fl ? *fl : trs::FrameList{});
     g_launches.fetch_add(1, std::memory_order_relaxed);
     CU(cudaGetLastError());
     return 0;
@@ -533,6 +561,7 @@ int trs_ctx_destroy(trs_ctx* ctx)
     cudaFree(ctx->frame_ctr);
     cudaFree(ctx->wp_dev); cudaFree(ctx->wp_grid_dev); cudaFree(ctx->wp_cells_dev); cudaFree(ctx->defer_dev);
     cudaFree(ctx->tk_desc); cudaFree(ctx->tk_scan); cudaFree(ctx->tk_grid); cudaFree(ctx->tk_cells); cudaFree(ctx->tk_scratch);
+    cudaFree(ctx->cfg_ctr); cudaFree(ctx->cfg_scratch);
     cudaFree(ctx->stats_dev);
     cudaFree(ctx->jpg_blob); cudaFree(ctx->jpg_planes); cudaFree(ctx->jpg_meta);
     cudaFree(ctx->jpe_meta); cudaFree(ctx->jpe_sizes); cudaFree(ctx->jpe_offs); cudaFree(ctx->jpe_blob);
@@ -566,6 +595,75 @@ int trs_preprocess(trs_ctx* ctx, const uint8_t* in_dev, int n, int h, int w, uin
     if (!in_dev) return fail(TRS_E_ARG, "null input");
     if (!out_u8_dev && !out_f32_dev && !stats_dev) return fail(TRS_E_ARG, "no output requested");
     return launch_preprocess(ctx, in_dev, n, h, w, out_u8_dev, out_f32_dev, stats_dev, nullptr, nullptr, false, (cudaStream_t)stream, 0);
+}
+
+int trs_set_preproc_configs(trs_ctx* ctx, const trs_preproc_params* cfgs, int n_cfgs)
+{
+    TRS_ENTER(ctx);
+    if (!cfgs) return fail(TRS_E_ARG, "null argument");
+    if (n_cfgs < 1 || n_cfgs > TRS_MAX_PREPROC_CONFIGS) return fail(TRS_E_ARG, "%d configurations, outside [1,%d]", n_cfgs, TRS_MAX_PREPROC_CONFIGS);
+    std::vector<trs::PreKParams> kp((size_t)n_cfgs);
+    for (int c = 0; c < n_cfgs; ++c) {
+        if (const int rc = derive_kparams(&cfgs[c], kp[(size_t)c])) {
+            char why[sizeof g_err];
+            snprintf(why, sizeof why, "%s", g_err);
+            return fail(rc, "configuration %d: %s", c, why);
+        }
+    }
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    if (!ctx->cfg_ctr) CU(cudaMalloc(&ctx->cfg_ctr, sizeof(uint32_t) * TRS_MAX_PREPROC_CONFIGS));
+    ctx->cfg_kp = std::move(kp);
+    ctx->n_cfgs = n_cfgs;
+    return 0;
+}
+
+int trs_preprocess_configs(trs_ctx* ctx, const uint8_t* in_dev, const int32_t* cfg_dev, int n, int h, int w, uint8_t* out_u8_dev, float* out_f32_dev,
+                           unsigned long long* stats_dev, void* stream)
+{
+    TRS_ENTER(ctx);
+    if (!ctx->n_cfgs) return fail(TRS_E_STATE, "trs_preprocess_configs before trs_set_preproc_configs");
+    if (n < 0 || h < 0 || w < 0) return fail(TRS_E_ARG, "negative size n=%d h=%d w=%d", n, h, w);
+    if (n == 0 || h == 0 || w == 0) return 0;
+    if (!in_dev || !cfg_dev) return fail(TRS_E_ARG, "null input");
+    if (!out_u8_dev && !out_f32_dev && !stats_dev) return fail(TRS_E_ARG, "no output requested");
+    const int k = ctx->n_cfgs;
+    cudaStream_t st = (cudaStream_t)stream;
+    std::lock_guard<std::mutex> lk(ctx->mu);
+    // bucket the frames by configuration without a sync (loc_tracks.cuh, as trs_locate_tracks buckets cars by track; preproc_list.h)
+    int chunk = 0, nblk = 0;
+    trs::loct_chunking(n, ctx->sm_count * 2, trs::LOCT_THREADS, chunk, nblk);
+    const size_t need = 1 + (size_t)(k + 2) + (size_t)(k + 1) * nblk + (size_t)n;
+    if (ctx->cfg_scratch_cap < need) {
+        cudaFree(ctx->cfg_scratch); ctx->cfg_scratch = nullptr; ctx->cfg_scratch_cap = 0;
+        CU(cudaMalloc(&ctx->cfg_scratch, sizeof(int) * need));
+        ctx->cfg_scratch_cap = need;
+    }
+    int* unused = ctx->cfg_scratch;                                  // (the walk's list counter that k_loct_scan clears)
+    int* start = unused + 1;
+    int* counts = start + (k + 2);
+    int* perm = counts + (size_t)(k + 1) * nblk;
+    CU(cudaMemsetAsync(ctx->cfg_ctr, 0, sizeof(uint32_t) * k, st));  // every configuration's frame tickets start at 0
+    trs::k_loct_hist<<<nblk, trs::LOCT_THREADS, sizeof(int) * (k + 1), st>>>(cfg_dev, n, k, chunk, nblk, counts, nullptr, nullptr);
+    trs::k_loct_scan<<<1, trs::LOCT_SCAN_THREADS, 0, st>>>(counts, nblk, k, n, start, unused);
+    trs::k_loct_scatter<<<nblk, trs::LOCT_THREADS, sizeof(int) * (k + 1) * (1 + trs::LOCT_THREADS / 32), st>>>(cfg_dev, n, k, chunk, nblk, counts, perm);
+    g_launches.fetch_add(3, std::memory_order_relaxed);
+    CU(cudaGetLastError());
+    // one launch per configuration, on the kernel trs_preprocess picks for it, over the configuration's slice of the permutation
+    for (int c = 0; c < k; ++c) {
+        trs::PreKParams kc = ctx->cfg_kp[(size_t)c];
+        kc.frame_ctr = ctx->cfg_ctr + c;
+        const trs::FrameList fl{perm, start, c};
+        const int rc = launch_preprocess(ctx, in_dev, n, h, w, out_u8_dev, out_f32_dev, stats_dev ? stats_dev + (size_t)c * TRS_STAT_COUNT : nullptr,
+                                         nullptr, nullptr, false, st, 0, &fl, &kc);
+        if (rc) return rc;
+    }
+    if (out_u8_dev || out_f32_dev) {
+        const trs::FrameList fl{perm, start, k};
+        trs::k_preprocess_unconfigured<<<std::min(n, ctx->sm_count * 4), trs::UNCFG_THREADS, 0, st>>>(fl, (size_t)h * w * 3, out_u8_dev, out_f32_dev);
+        g_launches.fetch_add(1, std::memory_order_relaxed);
+        CU(cudaGetLastError());
+    }
+    return 0;
 }
 
 int trs_debug_canny_stages(trs_ctx* ctx, const uint8_t* in_dev, int h, int w, uint16_t* mag_dev, uint8_t* map_dev, void* stream)
