@@ -1,6 +1,7 @@
-// Host build of the product's nearest-waypoint grid walk (csrc/loc_grid.h: the same source k_locate_grid and trs_set_track compile) for the
-// CPU-side parity test against the oracle (tests/test_host_logic.py).  Test infrastructure: mirrors trs_set_track + k_locate_grid + the
-// warp-per-car scan that finishes the cars the walk puts off, one car at a time.
+// Host build of the product's nearest-waypoint grid walk (csrc/loc_grid.h: the same source k_locate_grid and trs_set_track / trs_set_tracks
+// compile) for the CPU-side parity test against the oracle (tests/test_host_logic.py).  Test infrastructure: mirrors one track's table (the
+// distinct points and the grid loct_build makes of them for every track) + the walk + the warp-per-car scan that finishes the cars the walk
+// puts off, one car at a time; tests/host_locate_tracks_check.cpp runs the same walk over several tracks.
 #include "../triton-racer-sim_b200/csrc/loc_grid.h"
 using namespace trs;
 

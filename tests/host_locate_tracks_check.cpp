@@ -1,5 +1,5 @@
 // Host build of the multi-track nearest-waypoint path (csrc/loc_grid.h: the per-track tables trs_set_tracks uploads, the bucketing rules and the
-// slice / track selection of k_locate_tracks_grid) for the CPU-side tests (tests/test_locate_tracks_host.py).  Test infrastructure: restates the
+// slice / track selection of k_locate_grid<true>) for the CPU-side tests (tests/test_locate_tracks_host.py).  Test infrastructure: restates the
 // histogram / scan / scatter passes and the walk one car at a time, with the cars the walk puts off finished by the scan, as the kernels do.
 #include "../triton-racer-sim_b200/csrc/loc_grid.h"
 using namespace trs;
@@ -94,7 +94,7 @@ extern "C" int locate_tracks_host(const double* wp_cat, const int* n_wp, int k, 
             lo = end;
         }
     }
-    for (int car : list) {                                  // k_locate_tracks_warp: the track's distinct points in order of first occurrence, strict `<`
+    for (int car : list) {                                  // k_locate_warp<true>: the track's distinct points in order of first occurrence, strict `<`
         const LocTrack& d = h.desc[(size_t)trk[car]];
         const double* q = h.scan.data() + 4 * (size_t)d.scan_off;
         const double x = xyz[3 * (size_t)car], y = xyz[3 * (size_t)car + 1], z = xyz[3 * (size_t)car + 2];

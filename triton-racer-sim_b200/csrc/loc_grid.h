@@ -1,6 +1,7 @@
 // loc_grid.h — nearest waypoint through a uniform grid (track_data_process.py:89-107: L1 distance in float64, first index wins ties, the running
-// minimum starts at 100).  Pure host / device functions: k_locate_grid (misc_kernels.cuh) runs locg_walk per car, trs_set_track (trs_api.cu)
-// builds the table with locg_build, and tests/host_locate_check.cpp compiles the same source with g++ for the CPU-side parity test.
+// minimum starts at 100).  Pure host / device functions: k_locate_grid (misc_kernels.cuh) runs locg_walk per car, trs_set_track and trs_set_tracks
+// (trs_api.cu) build their tables with loct_build (one track or several), and tests/host_locate_check.cpp / host_locate_tracks_check.cpp compile
+// the same source with g++ for the CPU-side parity tests.
 //
 // The distinct points are bucketed into square cells of side c over (x, z).  c is a power of two, so floor(x / c) is exact and a point's and a
 // car's cell are decided by the same exact rule.  The points are sorted by cell (row-major, rows along z) behind a prefix array of cell starts.
@@ -206,11 +207,11 @@ inline std::vector<double> locg_distinct_quads(const double* wp, int n_wp)
     return quads;
 }
 
-// ---- several centre lines in one batch (trs_set_tracks / trs_locate_tracks, loc_tracks.cuh) ------------------------------------------------------
-// Every track keeps what trs_set_track builds for one: its distinct quads in order of first occurrence (the scan table) and, when locg_build gives
-// one, its cell-sorted quads and cell starts (the grid table).  The tracks' tables are concatenated; a descriptor per track holds the offsets.
-// Car i names its track t_i; the cars are bucketed by track (a stable counting sort) and each CTA of the walk takes a contiguous slice of the
-// bucketed cars, staging a track's grid table whenever its slice moves on to another track.
+// ---- the tables of one centre line or several (trs_set_track: k = 1, trs_set_tracks: k <= TRS_MAX_TRACKS) ----------------------------------------
+// Every track has its distinct quads in order of first occurrence (the scan table) and, when locg_build gives one, its cell-sorted quads and cell
+// starts (the grid table).  The tracks' tables are concatenated; a descriptor per track holds the offsets.  With several tracks car i names its
+// track t_i; the cars are bucketed by track (a stable counting sort) and each CTA of the walk takes a contiguous slice of the bucketed cars,
+// staging a track's grid table whenever its slice moves on to another track.  With one track the cars keep their own order.
 struct LocTrack {
     LocGrid g;                         // valid when grid_off >= 0
     double min_map, max_map;
@@ -230,8 +231,8 @@ struct LocTracksHost {
 };
 
 // Host: the tables of `k` centre lines (wp[t]: n_wp[t] x 3 f64).  A track whose grid would not fit `smem_limit` bytes, has non-finite
-// coordinates or fewer than LOCG_MIN_POINTS distinct points gets grid_off = -1.  Returns false when the concatenated tables would not be
-// addressable with int offsets.
+// coordinates or fewer than LOCG_MIN_POINTS distinct points gets grid_off = -1.  Returns false when a track's first quad in the concatenated
+// scan table would not be addressable with an int offset (never for the first track, so one centre line of any length is accepted).
 inline bool loct_build(const double* const* wp, const int* n_wp, const double* min_map, const double* max_map, int k, size_t smem_limit,
                        LocTracksHost& out)
 {
@@ -243,7 +244,7 @@ inline bool loct_build(const double* const* wp, const int* n_wp, const double* m
         const std::vector<double> quads = locg_distinct_quads(wp[t], n_wp[t]);
         d.min_map = min_map[t]; d.max_map = max_map[t];
         d.n_wp = n_wp[t]; d.n_u = (int)(quads.size() / 4);
-        if (out.scan.size() / 4 + quads.size() / 4 > (size_t)0x1fffffff) return false;
+        if (out.scan.size() / 4 > (size_t)0x1fffffff) return false;
         d.scan_off = (int)(out.scan.size() / 4);
         out.scan.insert(out.scan.end(), quads.begin(), quads.end());
         std::vector<double> sorted;
@@ -291,5 +292,15 @@ LOCG_HD int loct_track_of(const int* start, int k, int p)
     }
     return a;
 }
+
+#if defined(__CUDACC__)
+__device__ __forceinline__ double loct_nan() { return __longlong_as_double(0x7ff8000000000000LL); }
+
+// the reference's __map (track_data_process.py:105-107): idx / N * (max - min) + min, one rounding per operation
+__device__ __forceinline__ double loct_segment(int idx, int n_wp, double min_map, double max_map)
+{
+    return __dadd_rn(__dmul_rn(__ddiv_rn((double)idx, (double)n_wp), __dsub_rn(max_map, min_map)), min_map);
+}
+#endif
 
 }  // namespace trs

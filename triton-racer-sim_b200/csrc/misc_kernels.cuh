@@ -257,10 +257,7 @@ __global__ void __launch_bounds__(LOC_THREADS) k_locate(const double4* __restric
         const int k = base + c;
         if (k < n) {
             if (idx_out) idx_out[k] = (int)sel[c];
-            if (seg_out) {
-                const double q = __ddiv_rn(sel[c], (double)n_wp);
-                seg_out[k] = __dadd_rn(__dmul_rn(q, __dsub_rn(max_map, min_map)), min_map);
-            }
+            if (seg_out) seg_out[k] = loct_segment((int)sel[c], n_wp, min_map, max_map);
         }
     }
 }
@@ -289,26 +286,43 @@ __global__ void __launch_bounds__(PROBE64_THREADS) k_probe_fp64(double* __restri
 // (lane l takes waypoints l, l + 32, ...: ascending, so a lane keeps the first index of its own minimum) and a warp-shuffle
 // reduction on the pair (distance, index) — smaller distance, then smaller index — yields the reference's first-index argmin.
 // A thread per car would leave the GPU empty at these sizes.
+//
+// K6b and K6c serve one centre line (MULTI = false: trs_locate, the track's LocTrack `one` in the constant bank, no track index) and several
+// (MULTI = true: trs_locate_tracks, car i on track trk[i] with the descriptors `desc` and the scan table `scan` of loc_grid.h's loct_build).
 enum { LOCW_THREADS = 256 };
 
-// list != nullptr: the cars are list[0 .. *count) (the ones k_locate_grid put off), not 0 .. n.
-__global__ void __launch_bounds__(LOCW_THREADS) k_locate_warp(const double4* __restrict__ wp, int n_u, int n_wp, double min_map, double max_map,
-                                                              const double* __restrict__ xyz, int n, int32_t* __restrict__ idx_out,
+// list == nullptr: cars 0 .. n (with MULTI an out-of-range track index gets -1 / NaN); otherwise the cars list[0 .. *count) that k_locate_grid
+// put off (all in range).
+template <bool MULTI>
+__global__ void __launch_bounds__(LOCW_THREADS) k_locate_warp(const __grid_constant__ LocTrack one, const LocTrack* __restrict__ desc, int k,
+                                                              const double* __restrict__ scan, const double* __restrict__ xyz,
+                                                              const int32_t* __restrict__ trk, int n, int32_t* __restrict__ idx_out,
                                                               double* __restrict__ seg_out, const int* __restrict__ list = nullptr,
                                                               const int* __restrict__ count = nullptr)
 {
     const int lane = threadIdx.x & 31;
     const int warps_per_grid = (gridDim.x * blockDim.x) >> 5;
     if (list) n = *count;
-    for (int t = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; t < n; t += warps_per_grid) {
-        const int k = list ? list[t] : t;
-        const double px = xyz[3 * (size_t)k], py = xyz[3 * (size_t)k + 1], pz = xyz[3 * (size_t)k + 2];
+    for (int w = (blockIdx.x * blockDim.x + threadIdx.x) >> 5; w < n; w += warps_per_grid) {
+        const int car = list ? list[w] : w;
+        const int t = MULTI ? trk[car] : 0;
+        if (MULTI && (uint32_t)t >= (uint32_t)k) {
+            if (lane == 0) {
+                if (idx_out) idx_out[car] = -1;
+                if (seg_out) seg_out[car] = loct_nan();
+            }
+            continue;
+        }
+        const LocTrack& d = MULTI ? desc[t] : one;
+        const int n_u = d.n_u;
+        const double4* wp = reinterpret_cast<const double4*>(scan) + (MULTI ? d.scan_off : 0);     // (one track: scan_off is 0)
+        const double px = xyz[3 * (size_t)car], py = xyz[3 * (size_t)car + 1], pz = xyz[3 * (size_t)car + 2];
         double best = 100.0;                                     // track_data_process.py:93: the running minimum starts at 100
         int sel = 0x7fffffff;                                    // "nothing closer than 100 yet"
         for (int i = lane; i < n_u; i += 32) {
             const double2 qa = __ldg(reinterpret_cast<const double2*>(wp + i)), qb = __ldg(reinterpret_cast<const double2*>(wp + i) + 1);
-            const double d = __dadd_rn(__dadd_rn(fabs(__dsub_rn(px, qa.x)), fabs(__dsub_rn(py, qa.y))), fabs(__dsub_rn(pz, qb.x)));
-            if (d < best) { best = d; sel = (int)qb.y; }           // original indices ascend with i: a lane keeps the first index of its own minimum
+            const double dd = __dadd_rn(__dadd_rn(fabs(__dsub_rn(px, qa.x)), fabs(__dsub_rn(py, qa.y))), fabs(__dsub_rn(pz, qb.x)));
+            if (dd < best) { best = dd; sel = (int)qb.y; }       // original indices ascend with i: a lane keeps the first index of its own minimum
         }
 #pragma unroll
         for (int o = 16; o; o >>= 1) {
@@ -318,46 +332,78 @@ __global__ void __launch_bounds__(LOCW_THREADS) k_locate_warp(const double4* __r
         }
         if (lane == 0) {
             const int idx = sel == 0x7fffffff ? 0 : sel;        // nothing closer than 100: index 0 (:91-92)
-            if (idx_out) idx_out[k] = idx;
-            if (seg_out) {
-                const double q = __ddiv_rn((double)idx, (double)n_wp);
-                seg_out[k] = __dadd_rn(__dmul_rn(q, __dsub_rn(max_map, min_map)), min_map);
-            }
+            if (idx_out) idx_out[car] = idx;
+            if (seg_out) seg_out[car] = loct_segment(idx, d.n_wp, d.min_map, d.max_map);
         }
     }
 }
 
 // K6c: the same argmin through a uniform grid over (x, z): LARGE batches.  The algorithm and why it returns the reference's index bit for bit are in
-// loc_grid.h (host / device functions, also compiled by the CPU-side test): ~40 distance evaluations per car instead of ~1,000.  A car that has not
-// settled after the 3 x 3 block and LOCG_MAX_RINGS rings (far from the line but inside its bounding box) is appended to a list for the warp-per-car
-// kernel, so one such car never holds its warp for a scan of the whole grid.  Table in shared memory: quads in cell order + cell starts;
-// persistent CTAs, cars by grid stride.
+// loc_grid.h (host / device functions, also compiled by the CPU-side tests): ~40 distance evaluations per car instead of ~1,000.  A car that has not
+// settled after the 3 x 3 block and LOCG_MAX_RINGS rings (far from the line but inside its bounding box) is appended to a list for k_locate_warp,
+// so one such car never holds its warp for a scan of the whole grid.  Persistent CTAs; each stages the track's table (quads in cell order + cell
+// starts) in dynamic shared memory, sized for the largest table of the set.
+// One track: the cars 0 .. n by grid stride (contiguous slices per CTA measured 1-2 % slower on the shipped lines: neighbouring cars cost
+// alike, so one CTA can draw the expensive part of the line), the table is staged once and the LocTrack is read from the constant bank.  No
+// minimum-CTA bound (0): its 40 registers give 6 CTAs per SM anyway, and a bound of 6 makes ptxas move the cell-start base and the grid width
+// out of uniform registers, which measured 1 % slower on mountain_track.
+// Several tracks: CTA b takes positions loct_slice(start[k], b, gridDim.x) of the bucketed cars perm (k_loct_scatter, loc_tracks.cuh), splits its
+// slice at track boundaries and restages a track's table when the slice moves on to it; cars of a track without a grid go to the list whole.
+// The track's LocTrack lives in shared memory and ptxas keeps its fields in registers: bounded at 3 CTAs per SM it takes 74 registers without
+// spilling (by default it stops at 64 and spills).
 // ------------------------------------------------------------------------------------------------------
 enum { LOCG_THREADS = 256 };
 
-__global__ void __launch_bounds__(LOCG_THREADS) k_locate_grid(const double* __restrict__ quads, const int* __restrict__ cell_start, const LocGrid G, int n_wp,
-                                                              double min_map, double max_map, const double* __restrict__ xyz, int n,
-                                                              int32_t* __restrict__ idx_out, double* __restrict__ seg_out, int* __restrict__ defer_list,
-                                                              int* __restrict__ defer_count)
+template <bool MULTI>
+__global__ void __launch_bounds__(LOCG_THREADS, MULTI ? 3 : 0) k_locate_grid(const __grid_constant__ LocTrack one, const LocTrack* __restrict__ desc,
+                                                                          int k, const double* __restrict__ grid, const int* __restrict__ cells,
+                                                                          const int* __restrict__ start, const int* __restrict__ perm, int n,
+                                                                          const double* __restrict__ xyz, int32_t* __restrict__ idx_out,
+                                                                          double* __restrict__ seg_out, int* __restrict__ defer_list,
+                                                                          int* __restrict__ defer_count)
 {
     extern __shared__ __align__(16) uint8_t locg_smem[];
+    __shared__ LocTrack s_d;
     double* s_q = reinterpret_cast<double*>(locg_smem);
-    int* s_cs = reinterpret_cast<int*>(locg_smem + sizeof(double) * 4 * (size_t)G.n_u);
-    const int ncell = G.nx * G.nz;
-    for (int i = threadIdx.x; i < G.n_u; i += LOCG_THREADS) reinterpret_cast<double4*>(s_q)[i] = reinterpret_cast<const double4*>(quads)[i];
-    for (int i = threadIdx.x; i <= ncell; i += LOCG_THREADS) s_cs[i] = cell_start[i];
-    __syncthreads();
-    for (int k = blockIdx.x * LOCG_THREADS + threadIdx.x; k < n; k += gridDim.x * LOCG_THREADS) {
-        const int idx = locg_walk(G, s_q, s_cs, xyz[3 * (size_t)k], xyz[3 * (size_t)k + 1], xyz[3 * (size_t)k + 2]);
-        if (idx == LOCG_DEFERRED) {
-            defer_list[atomicAdd(defer_count, 1)] = k;
+    const int* s_cs = nullptr;
+    int lo, hi;
+    if (MULTI) loct_slice(start[k], blockIdx.x, gridDim.x, lo, hi);
+    else { lo = blockIdx.x * LOCG_THREADS; hi = n; }
+    const int stride = MULTI ? LOCG_THREADS : gridDim.x * LOCG_THREADS;
+    int staged = -1;
+    while (lo < hi) {
+        const int t = MULTI ? loct_track_of(start, k, lo) : 0;
+        const int end = MULTI ? min(hi, start[t + 1]) : hi;
+        const LocTrack& d = MULTI ? desc[t] : one;
+        if (MULTI && d.grid_off < 0) {                           // no grid for this track: every car to the scan
+            for (int p = lo + threadIdx.x; p < end; p += LOCG_THREADS) defer_list[atomicAdd(defer_count, 1)] = perm[p];
+            lo = end;
             continue;
         }
-        if (idx_out) idx_out[k] = idx;
-        if (seg_out) {
-            const double q = __ddiv_rn((double)idx, (double)n_wp);
-            seg_out[k] = __dadd_rn(__dmul_rn(q, __dsub_rn(max_map, min_map)), min_map);
+        if (t != staged) {
+            if (MULTI) __syncthreads();                          // every thread is done with the previous table (one track: there is none)
+            const int nu = d.g.n_u, ncell = d.g.nx * d.g.nz;
+            const double4* src = reinterpret_cast<const double4*>(grid) + (MULTI ? d.grid_off : 0);      // (one track: the offsets are 0)
+            for (int i = threadIdx.x; i < nu; i += LOCG_THREADS) reinterpret_cast<double4*>(s_q)[i] = src[i];
+            int* cs = reinterpret_cast<int*>(locg_smem + sizeof(double) * 4 * (size_t)nu);
+            for (int i = threadIdx.x; i <= ncell; i += LOCG_THREADS) cs[i] = cells[(MULTI ? d.cell_off : 0) + i];
+            if (MULTI && threadIdx.x == 0) s_d = d;
+            s_cs = cs;
+            staged = t;
+            __syncthreads();
         }
+        const LocTrack& e = MULTI ? s_d : one;
+        for (int p = lo + threadIdx.x; p < end; p += stride) {
+            const int car = MULTI ? perm[p] : p;
+            const int idx = locg_walk(e.g, s_q, s_cs, xyz[3 * (size_t)car], xyz[3 * (size_t)car + 1], xyz[3 * (size_t)car + 2]);
+            if (idx == LOCG_DEFERRED) {
+                defer_list[atomicAdd(defer_count, 1)] = car;
+                continue;
+            }
+            if (idx_out) idx_out[car] = idx;
+            if (seg_out) seg_out[car] = loct_segment(idx, e.n_wp, e.min_map, e.max_map);
+        }
+        lo = end;
     }
 }
 

@@ -75,6 +75,20 @@ struct TrsSwitches {
     size_t host_chunk_bytes = (size_t)48 << 20;      // ~48 MB of frames per chunk of the host pipeline (the link saturates from ~16 MB up)
 };
 
+// The device tables of one centre line (trs_set_track) or several (trs_set_tracks) as loct_build lays them out (loc_grid.h), and the scratch of
+// their large-batch path.
+struct LocSet {
+    int n_tracks = 0;                  // 0: no tables (none set yet, or the last upload failed)
+    trs::LocTrack* desc = nullptr;
+    double* scan = nullptr;            // distinct quads of every track in order of first occurrence
+    double* grid = nullptr;            // cell-sorted quads of the tracks that have a grid, nullptr: none has
+    int* cells = nullptr;
+    size_t smem = 0;                   // the largest grid table (dynamic shared memory of k_locate_grid)
+    trs::LocTrack one{};               // desc[0] on the host: the single-track kernels take it as a parameter
+    int* scratch = nullptr;            // [0] list count | several tracks: bucket starts (K + 2) | counts ((K + 1) x blocks) | bucketed cars (N) | list (N)
+    size_t scratch_cap = 0;            // ints
+};
+
 struct trs_ctx {
     int device = 0;
     TrsSwitches sw;
@@ -87,25 +101,8 @@ struct trs_ctx {
     trs_preproc_params user{};
     trs::PreKParams kp{};              // derived, geometry fields filled per call
     uint32_t* frame_ctr = nullptr;     // frame tickets of the store-warp kernels, one per launch slot: [0] trs_preprocess, [1 + s] staging set s
-    // track
-    double* wp_dev = nullptr;          // distinct waypoints in order of first occurrence: (x, y, z, original index) quads
-    int n_wp = 0, n_wp_distinct = 0;
-    double* wp_grid_dev = nullptr;     // the same quads sorted by grid cell (k_locate_grid), nullptr: no grid for this centre line
-    int* wp_cells_dev = nullptr;       // start of every cell in wp_grid_dev, ncell + 1 entries
-    trs::LocGrid grid{};
-    int* defer_dev = nullptr;          // [0] = count, [1 ..] = cars k_locate_grid left to the warp-per-car kernel
-    size_t defer_cap = 0;              // cars the list can hold
-    double min_map = 0, max_map = 10;
-    // several tracks (trs_set_tracks / trs_locate_tracks, loc_tracks.cuh): concatenated tables, a descriptor per track, and the scratch of the
-    // large-batch path
-    int n_tracks = 0;
-    trs::LocTrack* tk_desc = nullptr;
-    double* tk_scan = nullptr;         // distinct quads of every track in order of first occurrence
-    double* tk_grid = nullptr;         // cell-sorted quads of the tracks that have a grid, nullptr: none has
-    int* tk_cells = nullptr;
-    size_t tk_smem = 0;                // the largest grid table (dynamic shared memory of k_locate_tracks_grid)
-    int* tk_scratch = nullptr;         // [0] list count | bucket starts (K + 2) | counts ((K + 1) x blocks) | bucketed cars (N) | list (N)
-    size_t tk_scratch_cap = 0;         // ints
+    // nearest waypoint: the centre line of trs_set_track / trs_locate, and the ones of trs_set_tracks / trs_locate_tracks
+    LocSet track, tracks;
     // several preprocessing configurations (trs_set_preproc_configs / trs_preprocess_configs): the derived sets, a frame counter per
     // configuration, and the bucketing scratch: [0] unused count | bucket starts (K + 2) | counts ((K + 1) x blocks) | bucketed frames (N)
     int n_cfgs = 0;
@@ -483,6 +480,42 @@ int launch_preprocess(trs_ctx* ctx, const uint8_t* in, int n, int h, int w, uint
     return 0;
 }
 
+// device ints that grow on demand; the capacity is only recorded once the allocation succeeded
+int grow_ints(int*& buf, size_t& cap, size_t need)
+{
+    if (cap >= need) return 0;
+    cudaFree(buf); buf = nullptr; cap = 0;
+    CU(cudaMalloc(&buf, sizeof(int) * need));
+    cap = need;
+    return 0;
+}
+
+// Replaces the tables of s with h.  The set reads as empty from the first free until everything is uploaded, so a failed allocation or copy
+// can never leave tables of one upload next to those of another.
+template <bool MULTI>
+int upload_tracks(trs_ctx* ctx, LocSet& s, const trs::LocTracksHost& h)
+{
+    s.n_tracks = 0;
+    cudaFree(s.desc); cudaFree(s.scan); cudaFree(s.grid); cudaFree(s.cells);
+    s.desc = nullptr; s.scan = nullptr; s.grid = nullptr; s.cells = nullptr;
+    CU(cudaMalloc(&s.desc, sizeof(trs::LocTrack) * h.desc.size()));
+    CU(cudaMemcpy(s.desc, h.desc.data(), sizeof(trs::LocTrack) * h.desc.size(), cudaMemcpyHostToDevice));
+    CU(cudaMalloc(&s.scan, sizeof(double) * h.scan.size()));
+    CU(cudaMemcpy(s.scan, h.scan.data(), sizeof(double) * h.scan.size(), cudaMemcpyHostToDevice));
+    if (!h.grid.empty()) {
+        CU(cudaMalloc(&s.grid, sizeof(double) * h.grid.size()));
+        CU(cudaMemcpy(s.grid, h.grid.data(), sizeof(double) * h.grid.size(), cudaMemcpyHostToDevice));
+        CU(cudaMalloc(&s.cells, sizeof(int) * h.cells.size()));
+        CU(cudaMemcpy(s.cells, h.cells.data(), sizeof(int) * h.cells.size(), cudaMemcpyHostToDevice));
+        // the bound every table is built under, not this set's largest: the attribute belongs to the kernel, and other contexts may hold larger tables
+        CU(cudaFuncSetAttribute(trs::k_locate_grid<MULTI>, cudaFuncAttributeMaxDynamicSharedMemorySize, ctx->smem_optin - 1024));
+    }
+    s.smem = h.smem;
+    s.one = h.desc[0];
+    s.n_tracks = (int)h.desc.size();
+    return 0;
+}
+
 // staging buffers of the host pipeline grow on demand; the capacity is only recorded once all buffers of a kind exist, so a failed
 // allocation can never leave a stale capacity next to a null pointer
 template <class T>
@@ -559,8 +592,7 @@ int trs_ctx_destroy(trs_ctx* ctx)
     }
     if (ctx->host_entry) cudaEventDestroy(ctx->host_entry);
     cudaFree(ctx->frame_ctr);
-    cudaFree(ctx->wp_dev); cudaFree(ctx->wp_grid_dev); cudaFree(ctx->wp_cells_dev); cudaFree(ctx->defer_dev);
-    cudaFree(ctx->tk_desc); cudaFree(ctx->tk_scan); cudaFree(ctx->tk_grid); cudaFree(ctx->tk_cells); cudaFree(ctx->tk_scratch);
+    for (LocSet* s : {&ctx->track, &ctx->tracks}) { cudaFree(s->desc); cudaFree(s->scan); cudaFree(s->grid); cudaFree(s->cells); cudaFree(s->scratch); }
     cudaFree(ctx->cfg_ctr); cudaFree(ctx->cfg_scratch);
     cudaFree(ctx->stats_dev);
     cudaFree(ctx->jpg_blob); cudaFree(ctx->jpg_planes); cudaFree(ctx->jpg_meta);
@@ -632,12 +664,7 @@ int trs_preprocess_configs(trs_ctx* ctx, const uint8_t* in_dev, const int32_t* c
     // bucket the frames by configuration without a sync (loc_tracks.cuh, as trs_locate_tracks buckets cars by track; preproc_list.h)
     int chunk = 0, nblk = 0;
     trs::loct_chunking(n, ctx->sm_count * 2, trs::LOCT_THREADS, chunk, nblk);
-    const size_t need = 1 + (size_t)(k + 2) + (size_t)(k + 1) * nblk + (size_t)n;
-    if (ctx->cfg_scratch_cap < need) {
-        cudaFree(ctx->cfg_scratch); ctx->cfg_scratch = nullptr; ctx->cfg_scratch_cap = 0;
-        CU(cudaMalloc(&ctx->cfg_scratch, sizeof(int) * need));
-        ctx->cfg_scratch_cap = need;
-    }
+    if (const int rc = grow_ints(ctx->cfg_scratch, ctx->cfg_scratch_cap, 1 + (size_t)(k + 2) + (size_t)(k + 1) * nblk + (size_t)n)) return rc;
     int* unused = ctx->cfg_scratch;                                  // (the walk's list counter that k_loct_scan clears)
     int* start = unused + 1;
     int* counts = start + (k + 2);
@@ -737,86 +764,55 @@ int trs_set_track(trs_ctx* ctx, const double* wp_xyz_host, int n_wp, double min_
 {
     TRS_ENTER(ctx);
     if (!wp_xyz_host || n_wp <= 0) return fail(TRS_E_ARG, "empty centre line");
+    // only first occurrences are uploaded, each with its original index, and a uniform grid over (x, z) for k_locate_grid where one fits (loc_grid.h);
+    // none for non-finite coordinates, a handful of points or a table beyond shared memory: the scanning kernels serve every batch then
+    trs::LocTracksHost h;
+    trs::loct_build(&wp_xyz_host, &n_wp, &min_map, &max_map, 1, (size_t)ctx->smem_optin - 1024, h);      // (never refuses a first track)
     std::lock_guard<std::mutex> lk(ctx->mu);
-    // only first occurrences are uploaded, each with its original index (loc_grid.h)
-    const std::vector<double> quads = trs::locg_distinct_quads(wp_xyz_host, n_wp);
-    cudaFree(ctx->wp_dev);
-    ctx->wp_dev = nullptr;
-    CU(cudaMalloc(&ctx->wp_dev, sizeof(double) * quads.size()));
-    CU(cudaMemcpy(ctx->wp_dev, quads.data(), sizeof(double) * quads.size(), cudaMemcpyHostToDevice));
-    ctx->n_wp = n_wp;
-    ctx->n_wp_distinct = (int)(quads.size() / 4);
-    ctx->min_map = min_map;
-    ctx->max_map = max_map;
-    // uniform grid over (x, z) for k_locate_grid (loc_grid.h); none for non-finite coordinates, a handful of points or a table beyond shared memory:
-    // the scanning kernels serve every batch then
-    cudaFree(ctx->wp_grid_dev); ctx->wp_grid_dev = nullptr;
-    cudaFree(ctx->wp_cells_dev); ctx->wp_cells_dev = nullptr;
-    trs::LocGrid g{};
-    std::vector<double> sorted;
-    std::vector<int> start;
-    if (trs::locg_build(quads, (size_t)ctx->smem_optin - 1024, g, sorted, start)) {
-        CU(cudaMalloc(&ctx->wp_grid_dev, sizeof(double) * sorted.size()));
-        CU(cudaMemcpy(ctx->wp_grid_dev, sorted.data(), sizeof(double) * sorted.size(), cudaMemcpyHostToDevice));
-        CU(cudaMalloc(&ctx->wp_cells_dev, sizeof(int) * start.size()));
-        CU(cudaMemcpy(ctx->wp_cells_dev, start.data(), sizeof(int) * start.size(), cudaMemcpyHostToDevice));
-        // the bound every table is built under, not this table's size: the attribute belongs to the kernel, and another context's table may be larger
-        CU(cudaFuncSetAttribute(trs::k_locate_grid, cudaFuncAttributeMaxDynamicSharedMemorySize, ctx->smem_optin - 1024));
-        ctx->grid = g;
-    }
-    return 0;
+    return upload_tracks<false>(ctx, ctx->track, h);
 }
 
 int trs_locate(trs_ctx* ctx, const double* xyz_dev, int n, int32_t* idx_dev, double* segment_dev, void* stream)
 {
     TRS_ENTER(ctx);
-    if (!ctx->wp_dev) return fail(TRS_E_STATE, "trs_locate before trs_set_track");
+    if (!ctx->track.n_tracks) return fail(TRS_E_STATE, "trs_locate before trs_set_track");
     if (n < 0) return fail(TRS_E_ARG, "negative n");
     if (n == 0) return 0;
     if (!xyz_dev || (!idx_dev && !segment_dev)) return fail(TRS_E_ARG, "null pointer");
+    LocSet& s = ctx->track;
+    cudaStream_t st = (cudaStream_t)stream;
     // small batches: a warp per car with a shuffle reduction (a thread per car would not fill the GPU); large ones: the grid walk, with the
     // cars it puts off finished by the warp-per-car kernel; TRS_LOCATE=warp|thread|grid forces one
     const bool warp_per_car = ctx->sw.locate ? ctx->sw.locate == 1 : n < ctx->sm_count * 256;      // measured crossover ~50 k cars (15 us vs 55 us below it)
-    if (!warp_per_car && ctx->sw.locate != 2 && ctx->wp_grid_dev) {
+    if (!warp_per_car && ctx->sw.locate != 2 && s.grid) {
         std::lock_guard<std::mutex> lk(ctx->mu);
-        if (ctx->defer_cap < (size_t)n) {
-            cudaFree(ctx->defer_dev); ctx->defer_dev = nullptr; ctx->defer_cap = 0;
-            CU(cudaMalloc(&ctx->defer_dev, sizeof(int) * ((size_t)n + 1)));
-            ctx->defer_cap = (size_t)n;
-        }
-        cudaStream_t st = (cudaStream_t)stream;
-        CU(cudaMemsetAsync(ctx->defer_dev, 0, sizeof(int), st));
-        const trs::LocGrid& g = ctx->grid;
-        const size_t smem = trs::locg_table_bytes(g);
+        if (const int rc = grow_ints(s.scratch, s.scratch_cap, (size_t)n + 1)) return rc;
+        CU(cudaMemsetAsync(s.scratch, 0, sizeof(int), st));
         int per_sm = 0;
-        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, trs::k_locate_grid, trs::LOCG_THREADS, smem));
+        CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, trs::k_locate_grid<false>, trs::LOCG_THREADS, s.smem));
         per_sm = std::max(1, per_sm);
-        int grid = (n + trs::LOCG_THREADS - 1) / trs::LOCG_THREADS;
-        grid = std::min(grid, ctx->sm_count * per_sm);
-        trs::k_locate_grid<<<grid, trs::LOCG_THREADS, smem, st>>>(ctx->wp_grid_dev, ctx->wp_cells_dev, g, ctx->n_wp, ctx->min_map,
-                                                                  ctx->max_map, xyz_dev, n, idx_dev, segment_dev, ctx->defer_dev + 1, ctx->defer_dev);
+        const int grid = std::min((n + trs::LOCG_THREADS - 1) / trs::LOCG_THREADS, ctx->sm_count * per_sm);
+        trs::k_locate_grid<false><<<grid, trs::LOCG_THREADS, s.smem, st>>>(s.one, nullptr, 1, s.grid, s.cells, nullptr, nullptr, n, xyz_dev, idx_dev,
+                                                                           segment_dev, s.scratch + 1, s.scratch);
         CU(cudaGetLastError());
-        trs::k_locate_warp<<<ctx->sm_count * 2, trs::LOCW_THREADS, 0, st>>>(reinterpret_cast<const double4*>(ctx->wp_dev), ctx->n_wp_distinct, ctx->n_wp, ctx->min_map,
-                                                                            ctx->max_map, xyz_dev, n, idx_dev, segment_dev, ctx->defer_dev + 1, ctx->defer_dev);
+        trs::k_locate_warp<false><<<ctx->sm_count * 2, trs::LOCW_THREADS, 0, st>>>(s.one, nullptr, 1, s.scan, xyz_dev, nullptr, n, idx_dev, segment_dev,
+                                                                                   s.scratch + 1, s.scratch);
         g_launches.fetch_add(2, std::memory_order_relaxed);
         CU(cudaGetLastError());
         return 0;
     }
     if (warp_per_car) {
         const int warps_per_block = trs::LOCW_THREADS / 32;
-        int grid = (n + warps_per_block - 1) / warps_per_block;
-        const int cap = ctx->sm_count * 8;
-        if (grid > cap) grid = cap;
-        trs::k_locate_warp<<<grid, trs::LOCW_THREADS, 0, (cudaStream_t)stream>>>(reinterpret_cast<const double4*>(ctx->wp_dev), ctx->n_wp_distinct, ctx->n_wp,
-                                                                                 ctx->min_map, ctx->max_map, xyz_dev, n, idx_dev, segment_dev);
+        const int grid = std::min((n + warps_per_block - 1) / warps_per_block, ctx->sm_count * 8);
+        trs::k_locate_warp<false><<<grid, trs::LOCW_THREADS, 0, st>>>(s.one, nullptr, 1, s.scan, xyz_dev, nullptr, n, idx_dev, segment_dev);
         g_launches.fetch_add(1, std::memory_order_relaxed);
         CU(cudaGetLastError());
         return 0;
     }
     const int per_block = trs::LOC_THREADS * trs::LOC_CARS;
     const int grid = (n + per_block - 1) / per_block;
-    trs::k_locate<<<grid, trs::LOC_THREADS, 0, (cudaStream_t)stream>>>(reinterpret_cast<const double4*>(ctx->wp_dev), ctx->n_wp_distinct, ctx->n_wp, ctx->min_map,
-                                                                       ctx->max_map, xyz_dev, n, idx_dev, segment_dev);
+    trs::k_locate<<<grid, trs::LOC_THREADS, 0, st>>>(reinterpret_cast<const double4*>(s.scan), s.one.n_u, s.one.n_wp, s.one.min_map, s.one.max_map,
+                                                     xyz_dev, n, idx_dev, segment_dev);
     g_launches.fetch_add(1, std::memory_order_relaxed);
     CU(cudaGetLastError());
     return 0;
@@ -834,34 +830,18 @@ int trs_set_tracks(trs_ctx* ctx, const double* const* wp_xyz_host, const int* n_
     if (!trs::loct_build(wp_xyz_host, n_wp, min_map, max_map, n_tracks, (size_t)ctx->smem_optin - 1024, h))
         return fail(TRS_E_ARG, "centre lines too large for one table");
     std::lock_guard<std::mutex> lk(ctx->mu);
-    ctx->n_tracks = 0;                                               // (no tracks if an upload below fails)
-    cudaFree(ctx->tk_desc); cudaFree(ctx->tk_scan); cudaFree(ctx->tk_grid); cudaFree(ctx->tk_cells);
-    ctx->tk_desc = nullptr; ctx->tk_scan = nullptr; ctx->tk_grid = nullptr; ctx->tk_cells = nullptr;
-    CU(cudaMalloc(&ctx->tk_desc, sizeof(trs::LocTrack) * h.desc.size()));
-    CU(cudaMemcpy(ctx->tk_desc, h.desc.data(), sizeof(trs::LocTrack) * h.desc.size(), cudaMemcpyHostToDevice));
-    CU(cudaMalloc(&ctx->tk_scan, sizeof(double) * h.scan.size()));
-    CU(cudaMemcpy(ctx->tk_scan, h.scan.data(), sizeof(double) * h.scan.size(), cudaMemcpyHostToDevice));
-    if (!h.grid.empty()) {
-        CU(cudaMalloc(&ctx->tk_grid, sizeof(double) * h.grid.size()));
-        CU(cudaMemcpy(ctx->tk_grid, h.grid.data(), sizeof(double) * h.grid.size(), cudaMemcpyHostToDevice));
-        CU(cudaMalloc(&ctx->tk_cells, sizeof(int) * h.cells.size()));
-        CU(cudaMemcpy(ctx->tk_cells, h.cells.data(), sizeof(int) * h.cells.size(), cudaMemcpyHostToDevice));
-        // the bound every table is built under, not this set's largest: the attribute belongs to the kernel, and other contexts may hold larger tables
-        CU(cudaFuncSetAttribute(trs::k_locate_tracks_grid, cudaFuncAttributeMaxDynamicSharedMemorySize, ctx->smem_optin - 1024));
-    }
-    ctx->tk_smem = h.smem;
-    ctx->n_tracks = n_tracks;
-    return 0;
+    return upload_tracks<true>(ctx, ctx->tracks, h);
 }
 
 int trs_locate_tracks(trs_ctx* ctx, const double* xyz_dev, const int32_t* track_dev, int n, int32_t* idx_dev, double* segment_dev, void* stream)
 {
     TRS_ENTER(ctx);
-    if (!ctx->n_tracks) return fail(TRS_E_STATE, "trs_locate_tracks before trs_set_tracks");
+    if (!ctx->tracks.n_tracks) return fail(TRS_E_STATE, "trs_locate_tracks before trs_set_tracks");
     if (n < 0) return fail(TRS_E_ARG, "negative n");
     if (n == 0) return 0;
     if (!xyz_dev || !track_dev || (!idx_dev && !segment_dev)) return fail(TRS_E_ARG, "null pointer");
-    const int k = ctx->n_tracks;
+    LocSet& s = ctx->tracks;
+    const int k = s.n_tracks;
     cudaStream_t st = (cudaStream_t)stream;
     // small batches: a warp per car straight from the cars' order (the same crossover as trs_locate); large ones: bucket the cars by track, walk
     // the grids, finish the cars the walk puts off with a warp per car.  TRS_LOCATE=warp|thread|grid forces one (thread: a scan per bucketed car).
@@ -869,7 +849,7 @@ int trs_locate_tracks(trs_ctx* ctx, const double* xyz_dev, const int32_t* track_
     if (warp_per_car) {
         const int warps_per_block = trs::LOCW_THREADS / 32;
         const int grid = std::min((n + warps_per_block - 1) / warps_per_block, ctx->sm_count * 8);
-        trs::k_locate_tracks_warp<<<grid, trs::LOCW_THREADS, 0, st>>>(ctx->tk_desc, k, ctx->tk_scan, xyz_dev, track_dev, n, idx_dev, segment_dev);
+        trs::k_locate_warp<true><<<grid, trs::LOCW_THREADS, 0, st>>>(s.one, s.desc, k, s.scan, xyz_dev, track_dev, n, idx_dev, segment_dev);
         g_launches.fetch_add(1, std::memory_order_relaxed);
         CU(cudaGetLastError());
         return 0;
@@ -877,13 +857,8 @@ int trs_locate_tracks(trs_ctx* ctx, const double* xyz_dev, const int32_t* track_
     std::lock_guard<std::mutex> lk(ctx->mu);
     int chunk = 0, nblk = 0;
     trs::loct_chunking(n, ctx->sm_count * 2, trs::LOCT_THREADS, chunk, nblk);
-    const size_t need = 1 + (size_t)(k + 2) + (size_t)(k + 1) * nblk + 2 * (size_t)n;
-    if (ctx->tk_scratch_cap < need) {
-        cudaFree(ctx->tk_scratch); ctx->tk_scratch = nullptr; ctx->tk_scratch_cap = 0;
-        CU(cudaMalloc(&ctx->tk_scratch, sizeof(int) * need));
-        ctx->tk_scratch_cap = need;
-    }
-    int* count = ctx->tk_scratch;
+    if (const int rc = grow_ints(s.scratch, s.scratch_cap, 1 + (size_t)(k + 2) + (size_t)(k + 1) * nblk + 2 * (size_t)n)) return rc;
+    int* count = s.scratch;
     int* start = count + 1;
     int* counts = start + (k + 2);
     int* perm = counts + (size_t)(k + 1) * nblk;
@@ -895,20 +870,20 @@ int trs_locate_tracks(trs_ctx* ctx, const double* xyz_dev, const int32_t* track_
     CU(cudaGetLastError());
     if (ctx->sw.locate == 2) {
         const int grid = std::min((n + trs::LOCT_THREADS - 1) / trs::LOCT_THREADS, ctx->sm_count * 16);
-        trs::k_locate_tracks_scan<<<grid, trs::LOCT_THREADS, 0, st>>>(ctx->tk_desc, k, ctx->tk_scan, start, perm, xyz_dev, track_dev, idx_dev, segment_dev);
+        trs::k_locate_tracks_scan<<<grid, trs::LOCT_THREADS, 0, st>>>(s.desc, k, s.scan, start, perm, xyz_dev, track_dev, idx_dev, segment_dev);
         g_launches.fetch_add(1, std::memory_order_relaxed);
         CU(cudaGetLastError());
         return 0;
     }
     int per_sm = 0;
-    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, trs::k_locate_tracks_grid, trs::LOCG_THREADS, ctx->tk_smem));
+    CU(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, trs::k_locate_grid<true>, trs::LOCG_THREADS, s.smem));
     per_sm = std::max(1, per_sm);
     const int grid = std::min((n + trs::LOCG_THREADS - 1) / trs::LOCG_THREADS, ctx->sm_count * per_sm);
-    trs::k_locate_tracks_grid<<<grid, trs::LOCG_THREADS, ctx->tk_smem, st>>>(ctx->tk_desc, k, ctx->tk_grid, ctx->tk_cells, start, perm, xyz_dev,
-                                                                             idx_dev, segment_dev, list, count);
+    trs::k_locate_grid<true><<<grid, trs::LOCG_THREADS, s.smem, st>>>(s.one, s.desc, k, s.grid, s.cells, start, perm, n, xyz_dev, idx_dev, segment_dev,
+                                                                      list, count);
     CU(cudaGetLastError());
-    trs::k_locate_tracks_warp<<<ctx->sm_count * 2, trs::LOCW_THREADS, 0, st>>>(ctx->tk_desc, k, ctx->tk_scan, xyz_dev, track_dev, n, idx_dev,
-                                                                               segment_dev, list, count);
+    trs::k_locate_warp<true><<<ctx->sm_count * 2, trs::LOCW_THREADS, 0, st>>>(s.one, s.desc, k, s.scan, xyz_dev, track_dev, n, idx_dev, segment_dev,
+                                                                              list, count);
     g_launches.fetch_add(2, std::memory_order_relaxed);
     CU(cudaGetLastError());
     return 0;
